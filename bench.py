@@ -49,7 +49,32 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-post", action="store_true", help="skip the timing of the post-scan host steps")
     ap.add_argument("--no-extra", action="store_true", help="skip the stages reported beside the metric (wall time to links, C5 chain)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64; "
+                         "link tables as a fixed, seeded sample of rows) so that two builds can be compared output for output. "
+                         "The timed steps keep their link rows on the device: the rows written come from one more scan of the same "
+                         "inputs, whose counts, thresholds and probabilities must equal the last timed step's")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+DUMP_ROWS = 400_000  # rows sampled per link table: 2 tables x 8 float64 columns x 400k rows = 51 MB, under 64 MB in all
+LINK_COLS = ("pos1", "pos2", "clust1", "clust2", "len", "block", "MI")
+
+
+def sample_rows(n: int, k: int = DUMP_ROWS) -> np.ndarray:
+    """Row indices of a link table of n rows that --dump-outputs writes: all of them, or k drawn with a fixed seed (sorted)."""
+    if n <= k:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def load_peaks():
@@ -319,11 +344,13 @@ def main():
         for _ in range(args.steps):
             barrier()
             t0 = time.perf_counter()
-            grp.hdw(0.1)
+            w_last = grp.hdw(0.1)
             barrier()
             times.append(allmax(time.perf_counter() - t0))
         if rank != 0:
             return finish()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"hdw": w_last})
         ops = 5.0 * n * S * S  # SURVEY 8d: algorithmic int8 work of the five one-hot crossprods
         i8 = int8_peak_tops(torch.device("cuda", local_rank))
         pk = i8[0] if i8 else 2 * peaks["bf16_tflops"]
@@ -362,7 +389,7 @@ def main():
     stats = None
     agg = {"n_pairs": 0, "n_launches": 0, "n_scan_launches": 0, "exec_int8_ops": 0.0, "exec_mufu_ops": 0.0, "n_tiles": 0}
     for _ in range(args.steps):
-        *_, st_list = scan(flags_dev)
+        sr_n, lr_n, _, thr_last, prob_last, st_list = scan(flags_dev)
         stats = st_list[0]
         dev_ms += stats["t_scan_ms"] + stats["t_select_ms"]
         step_ms.append(stats["t_scan_ms"] + stats["t_select_ms"])
@@ -485,6 +512,26 @@ def main():
                     del res
         except Exception as ex:  # noqa: BLE001
             extra["error"] = repr(ex)
+
+    if args.dump_outputs:
+        # The timed steps leave their link columns in device memory (LDW_SCAN_NO_D2H).  One more scan of the same inputs
+        # copies them out; the scan is deterministic, and its counts, thresholds and probabilities must equal the last
+        # timed step's before its rows are written as that step's.
+        sr_d, lr_d, _, thr_d, prob_d, _ = scan(base_flags)
+        if rank == 0:
+            if (int(sr_d.n), int(lr_d.n)) != (int(sr_n.n), int(lr_n.n)) or not (
+                    np.array_equal(thr_d, thr_last, equal_nan=True) and np.array_equal(prob_d, prob_last, equal_nan=True)):
+                raise SystemExit("--dump-outputs: a repeated scan of the same inputs differs from the last timed step")
+            out = {"thr": thr_last, "prob": prob_last, "n_links": np.array([int(sr_n.n), int(lr_n.n)])}
+            for tag, tbl in (("sr", sr_d), ("lr", lr_d)):
+                rows = sample_rows(int(tbl.n))
+                cols = tbl.views()
+                if rows.size and set(LINK_COLS) - set(cols):
+                    raise SystemExit(f"--dump-outputs: {tag} link table lacks columns {sorted(set(LINK_COLS) - set(cols))}")
+                out[f"{tag}_rows"] = rows
+                for k in LINK_COLS:
+                    out[f"{tag}_{k}"] = cols[k][rows] if rows.size else np.zeros(0)
+            dump_outputs(args.dump_outputs, out)
 
     if rank != 0:
         return finish()

@@ -15,9 +15,12 @@ from hypothesis import strategies as st
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_golden_ref_cases as GC  # noqa: E402
 import ref_lib  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not built and /root/reference absent")
+HAVE_REF = ref_lib.available()
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref not built and the reference sources absent")
 
 
 def reference_view(path):
@@ -55,8 +58,24 @@ def product_view(path, chunk=None):
             os.environ["LDW_FASTA_CHUNK"] = old
 
 
-def check_same(path, chunk=None):
-    rnames, rseqs, _ = reference_view(path)
+GOLD = GC.load()
+
+
+def stored_views(group):
+    """The reference reader's (names, sequences) for each stored input of `group` (tests/golden/ref_cases.npz)."""
+    return list(zip(GC.get_lists(GOLD, group + "_names"), GC.get_lists(GOLD, group + "_seqs")))
+
+
+def expected_view(want, path):
+    """`want` (stored), checked against the compiled reader where it is built."""
+    if HAVE_REF:
+        names, seqs, _ = reference_view(path)
+        assert (names, seqs) == tuple(want), "tests/golden/ref_cases.npz differs from the compiled reader"
+    return want
+
+
+def check_same(path, want, chunk=None):
+    rnames, rseqs = want
     nseq, slen, names, aln = product_view(path, chunk)
     assert nseq == len(rseqs), (nseq, len(rseqs))
     assert names == rnames
@@ -107,52 +126,72 @@ CASES = {
 
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_reader_matches_kseq_on_handwritten_files(tmp_path, name):
+    i = sorted(CASES).index(name)
+    assert GC.get_lists(GOLD, "hand_in")[i] == [CASES[name]]
+    want = stored_views("hand")[i]
     p = tmp_path / (name + ".fa")
     p.write_bytes(CASES[name])
-    check_same(str(p))
+    expected_view(want, str(p))
+    check_same(str(p), want)
     for chunk in (1, 2, 3, 7):
-        check_same(str(p), chunk)
+        check_same(str(p), want, chunk)
     q = tmp_path / (name + ".fa.gz")
     with gzip.open(q, "wb") as fh:
         fh.write(CASES[name])
-    check_same(str(q))
+    expected_view(want, str(q))
+    check_same(str(q), want)
 
 
 def test_documented_semantics_are_the_references(tmp_path):
-    """The cases VERDICT/ADVICE name: the expected values come from the compiled kseq2.h, spelled out once here."""
+    """The cases VERDICT/ADVICE name: the expected values come from the compiled kseq2.h, spelled out once here.  The
+    reader is held to them everywhere; the compiled kseq2.h is checked against them too where it is built."""
     p = tmp_path / "crlf.fa"
     p.write_bytes(b">a\r\nACGT\r\nAC\r\n")
-    names, seqs, rc = reference_view(str(p))
-    assert (names, seqs, rc) == ([b"a"], [b"ACGT\rAC\r"], -1)     # seq.length 8, where a whitespace stripper gives 6
+    if HAVE_REF:
+        names, seqs, rc = reference_view(str(p))
+        assert (names, seqs, rc) == ([b"a"], [b"ACGT\rAC\r"], -1)     # seq.length 8, where a whitespace stripper gives 6
     assert product_view(str(p))[:2] == (1, 8)
+    assert product_view(str(p))[3] == b"ACGT\rAC\r"
     p.write_bytes(b">a\nACGT\n\n>b\nAC\n")
-    assert reference_view(str(p))[1] == [b"ACGT\n>bAC"]
+    if HAVE_REF:
+        assert reference_view(str(p))[1] == [b"ACGT\n>bAC"]
     assert product_view(str(p))[3] == b"ACGT\n>bAC"
+
+
+EDGE16K_TOTALS = (16384, 16383, 32768, 16385)
+
+
+def edge16k_stream(total):
+    body = b">a\n" + b"A" * (total - 3 - 2) + b"\n>"
+    assert len(body) == total
+    return body
 
 
 def test_header_char_as_last_byte_of_a_16384_multiple_stream(tmp_path):
     """ks_getuntil only knows EOF after a short read (src/kseq2.h:87-98): a lone '>' closing a stream whose length is a
     multiple of the 16384-byte buffer yields one more, empty, record; any other length yields none."""
-    for total in (16384, 16383, 32768, 16385):
-        body = b">a\n" + b"A" * (total - 3 - 2) + b"\n>"
-        assert len(body) == total
+    for total, want in zip(EDGE16K_TOTALS, stored_views("edge16k")):
         p = tmp_path / f"t{total}.fa"
-        p.write_bytes(body)
-        check_same(str(p))
-        check_same(str(p), 5)
+        p.write_bytes(edge16k_stream(total))
+        expected_view(want, str(p))
+        check_same(str(p), want)
+        check_same(str(p), want, 5)
 
 
 ALPHABET = [b">", b"@", b"+", b"\n", b"\n", b"\r", b" ", b"\t", b"A", b"c", b"N", b"-", b"\0", b"x"]
 
 
+@needs_ref
 @settings(max_examples=400, deadline=None, suppress_health_check=[HealthCheck.function_scoped_fixture])
 @given(data=st.lists(st.sampled_from(ALPHABET), min_size=0, max_size=60).map(b"".join), chunk=st.sampled_from([None, 1, 2, 5]))
 def test_reader_matches_kseq_on_random_byte_streams(tmp_path, data, chunk):
     p = tmp_path / "fuzz.fa"
     p.write_bytes(data)
-    check_same(str(p), chunk)
+    names, seqs, _ = reference_view(str(p))
+    check_same(str(p), (names, seqs), chunk)
 
 
+@needs_ref
 @settings(max_examples=150, deadline=None, suppress_health_check=[HealthCheck.function_scoped_fixture])
 @given(recs=st.lists(st.tuples(st.sampled_from([b">", b"@"]),
                                st.lists(st.sampled_from([b"ACGT", b"acgtn-", b"", b"AC GT", b"\r", b"+", b"II"]),
@@ -167,7 +206,20 @@ def test_reader_matches_kseq_on_record_shaped_streams(tmp_path, recs, chunk):
             out += ln + eol
     p = tmp_path / "fuzz2.fa"
     p.write_bytes(bytes(out))
-    check_same(str(p), chunk)
+    names, seqs, _ = reference_view(str(p))
+    check_same(str(p), (names, seqs), chunk)
+
+
+def test_reader_matches_kseq_on_a_stored_sample_of_random_streams(tmp_path):
+    """The two property tests above on a fixed seeded sample of their streams (make_golden_ref_cases.random_streams),
+    inputs and the reference reader's views stored: the comparison runs where the compiled reader is not built too."""
+    streams = [s[0] for s in GC.get_lists(GOLD, "random_in")]
+    assert streams == GC.random_streams(2024, len(streams))
+    for i, (data, want) in enumerate(zip(streams, stored_views("random"))):
+        p = tmp_path / "sample.fa"
+        p.write_bytes(data)
+        expected_view(want, str(p))
+        check_same(str(p), want, (None, 1, 2, 5)[i % 4])
 
 
 def test_two_call_reader_agrees_with_the_single_call_one(tmp_path):
@@ -185,27 +237,35 @@ def test_two_call_reader_agrees_with_the_single_call_one(tmp_path):
     assert bytes(aln[0]) == b"ACGT\rAC\r" and bytes(aln[1]) == b"TTTT\rGG\r" and names.raw.split(b"\0")[:2] == [b"a", b"b"]
 
 
+def crlf_alignment_file():
+    rng = np.random.default_rng(5)
+    nseq, L = 40, 300
+    base = rng.choice(list(b"ACGT"), size=L)
+    out = bytearray()
+    for k in range(nseq):
+        r = base.copy()
+        m = rng.random(L) < 0.2
+        r[m] = rng.choice(list(b"ACGTacgtN-"), size=int(m.sum()))
+        r = bytes(r.astype(np.uint8))
+        out += b">s%d\r\n" % k
+        for o in range(0, L, 70):
+            out += r[o:o + 70] + b"\r\n"
+    return bytes(out)
+
+
 def test_whole_encode_chain_on_a_crlf_alignment_matches_the_reference_host_side(tmp_path):
     """POS/seq.length after the tokeniser: the reference's extractAlnParam on a CRLF file counts the CR columns (class
     'other'); the product's reader must hand the same matrix to the device kernels (checked here on the host: the
     matrix bytes equal what kseq gives, and the oracle's filter on that matrix equals the reference's POS)."""
     import ldw_oracle as O
-    rng = np.random.default_rng(5)
-    nseq, L = 40, 300
-    base = rng.choice(list(b"ACGT"), size=L)
-    rows = []
-    for _ in range(nseq):
-        r = base.copy()
-        m = rng.random(L) < 0.2
-        r[m] = rng.choice(list(b"ACGTacgtN-"), size=int(m.sum()))
-        rows.append(bytes(r.astype(np.uint8)))
+    L = 300
     p = tmp_path / "crlf_aln.fa"
-    with open(p, "wb") as fh:
-        for k, r in enumerate(rows):
-            fh.write(b">s%d\r\n" % k)
-            for o in range(0, L, 70):
-                fh.write(r[o:o + 70] + b"\r\n")
-    ref = ref_lib.extractAlnParam(str(p), 0, 0.15, 0.01)
+    p.write_bytes(crlf_alignment_file())
+    ref = {"num.seqs": int(GOLD["crlf_shape"][0]), "seq.length": int(GOLD["crlf_shape"][1]), "pos": GOLD["crlf_pos"]}
+    if HAVE_REF:
+        live = ref_lib.extractAlnParam(str(p), 0, 0.15, 0.01)
+        assert (live["num.seqs"], live["seq.length"]) == (ref["num.seqs"], ref["seq.length"])
+        np.testing.assert_array_equal(live["pos"], ref["pos"])
     nseq_p, slen_p, names, aln = product_view(str(p))
     assert (nseq_p, slen_p) == (ref["num.seqs"], ref["seq.length"]) and slen_p == L + 5  # five CRs per record
     seqs = [aln[i * slen_p:(i + 1) * slen_p] for i in range(nseq_p)]
