@@ -351,9 +351,12 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
 #pragma unroll
     for (int b = 0; b < RB; b++) rbv[b] = __uint_as_float(rpj[jj][b]);
     // every marginal carries the pseudocounts of its row / column, so the corner comes out as count + M; the count
-    // itself can be slightly negative (floor semantics of the other cells): clamp it at zero
-    const int corner = (int)(k.Ti[PA] + tot[jj] - sj);
-    row[PB] = (uint32_t)max(corner, (int)k.M);
+    // itself can be slightly negative (floor semantics of the other cells): clamp it at zero.  Unsigned throughout: the
+    // corner can hold up to the whole table, i.e. 2^31 count units and more (the unit is sized so that a table fits
+    // 32 bits, not 31).  rest = sum_b (cell(PA, b) + M) >= 0: each of its terms is a complement, non-negative under
+    // floor semantics.
+    const uint32_t rest = sj - tot[jj];
+    row[PB] = k.Ti[PA] >= rest ? max(k.Ti[PA] - rest, k.M) : k.M;
     acc[jj] = mi_row<QC, RB>(acc[jj], row, k.rpad[PA], rbv, dq[jj]);
   }
   // ---- classification and emission: tile-uniform branches only; the per-lane work is predicated
