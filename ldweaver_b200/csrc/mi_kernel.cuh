@@ -148,6 +148,12 @@ __device__ __forceinline__ uint4 lds128(uint32_t saddr) {
   return v;
 }
 
+__device__ __forceinline__ uint2 lds64(uint32_t saddr) {
+  uint2 v;
+  asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(saddr));
+  return v;
+}
+
 __device__ __forceinline__ void sts128(uint32_t saddr, uint4 v) {
   asm volatile("st.shared.v4.u32 [%0], {%1, %2, %3, %4};" ::"r"(saddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
@@ -270,27 +276,39 @@ __device__ __forceinline__ void epi_load(uint32_t tmem_base, int NJ, int j0, uin
     }
 }
 
+// The PA x PB accumulator cells of a batch as counts in the count unit, pseudocount included.
+template <int PA, int PB, int JC>
+__device__ __forceinline__ void epi_counts(const uint32_t (&H)[PA][PB][JC], const uint32_t (&L)[PA][PB][JC], uint32_t mul_a,
+                                           uint32_t sb, uint32_t M, uint32_t (&T)[PA][PB][JC]) {
+#pragma unroll
+  for (int a = 0; a < PA; a++)
+#pragma unroll
+    for (int b = 0; b < PB; b++)
+#pragma unroll
+      for (int jj = 0; jj < JC; jj++) T[a][b][jj] = H[a][b][jj] * mul_a + ((L[a][b][jj] >> sb) + M);
+}
+
 // JC pairs (this thread's row SNP x JC column SNPs), evaluated in lock step: term loop outside, pair loop inside, so
-// JC independent dependency chains overlap each other's MUFU / conversion latency.
+// JC independent dependency chains overlap each other's MUFU / conversion latency.  T: the batch's counts (epi_counts).
 template <int PA, int PB, int JC, bool QC, bool RG>
 __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, const TileRegs<PA + 1>& k, int j0,
-                                          const uint32_t (&H)[PA][PB][JC], const uint32_t (&L)[PA][PB][JC]) {
+                                          const uint32_t (&T)[PA][PB][JC]) {
   constexpr int RB = PB + 1;
-  uint32_t tj[JC][RB], rpj[JC][RB];
+  uint32_t rpj[JC][RB];
   int jl[JC];
   float dq[JC];
-  uint4 d0v[JC];
 #pragma unroll
   for (int jj = 0; jj < JC; jj++) {
     const uint32_t ra_ = c.jrec_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(Rec);
-    const uint4 w0 = lds128(ra_), w1 = lds128(ra_ + (QC ? 32 : 16));  // T, then q (Q1 form) or rp (plain form)
-    uint4 w3 = make_uint4(0, 0, 0, 0);
-    if (RB == 5) w3 = lds128(ra_ + 48);
-    const uint32_t tt[5] = {w0.x, w0.y, w0.z, w0.w, w3.x}, tr[5] = {w1.x, w1.y, w1.z, w1.w, QC ? w3.z : w3.y};
+    const uint4 w1 = lds128(ra_ + (QC ? 32 : 16));  // q (Q1 form) or rp (plain form); the totals T at the last row
+    uint32_t w4 = 0;                                 // q4 / rp4
+    if (RB == 5) asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w4) : "r"(ra_ + (QC ? 56 : 52)));
+    const uint32_t tr[5] = {w1.x, w1.y, w1.z, w1.w, w4};
 #pragma unroll
-    for (int b = 0; b < RB; b++) { tj[jj][b] = tt[b]; rpj[jj][b] = tr[b]; }
-    d0v[jj] = lds128(c.jdyn_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(ColDyn));
-    jl[jj] = (int)d0v[jj].x;
+    for (int b = 0; b < RB; b++) rpj[jj][b] = tr[b];
+    // only .x (jl) and .y (the Q1 factor) are needed here; the short-range bounds in .z / .w are reloaded at emission
+    const uint2 d0 = lds64(c.jdyn_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(ColDyn));
+    jl[jj] = (int)d0.x;
     dq[jj] = 0.f;
     if (QC) {
       if (RG) {
@@ -303,7 +321,7 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
         }
         dq[jj] = v - k.q0;
       } else {
-        dq[jj] = fmaf(k.rtlq, __uint_as_float(d0v[jj].y), -k.q0);
+        dq[jj] = fmaf(k.rtlq, __uint_as_float(d0.y), -k.q0);
       }
     }
   }
@@ -326,7 +344,7 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
       uint32_t rsum = 0;
 #pragma unroll
       for (int b = 0; b < PB; b++) {
-        const uint32_t t = H[a][b][jj] * k.mul_a + ((L[a][b][jj] >> k.sb) + k.M);  // count + pseudocount
+        const uint32_t t = T[a][b][jj];
         rsum += t;
         col[jj][b] += t;
         row[jj][b] = t;
@@ -344,10 +362,12 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
   }
 #pragma unroll
   for (int jj = 0; jj < JC; jj++) {
+    const uint4 w0 = lds128(c.jrec_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(Rec));  // the column totals T
+    const uint32_t tj[4] = {w0.x, w0.y, w0.z, w0.w};
     uint32_t row[RB], sj = 0;
     float rbv[RB];
 #pragma unroll
-    for (int b = 0; b < PB; b++) { row[b] = tj[jj][b] - col[jj][b]; sj += tj[jj][b]; }
+    for (int b = 0; b < PB; b++) { row[b] = tj[b] - col[jj][b]; sj += tj[b]; }
 #pragma unroll
     for (int b = 0; b < RB; b++) rbv[b] = __uint_as_float(rpj[jj][b]);
     // every marginal carries the pseudocounts of its row / column, so the corner comes out as count + M; the count
@@ -375,7 +395,7 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
   if (k.has_sr) {
 #pragma unroll
     for (int jj = 0; jj < JC; jj++) {
-      const uint4 d0 = d0v[jj];
+      const uint4 d0 = lds128(c.jdyn_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(ColDyn));
       const uint4 d1 = lds128(c.jdyn_saddr + (uint32_t)(j0 + jj) * (uint32_t)sizeof(ColDyn) + 16);
       const uint32_t la = d0.w - d0.z, lb = d1.y - d1.x;
       const bool sr = live[jj] && (((uint32_t)k.il - d0.z < la) || ((uint32_t)k.il - d1.x < lb));
@@ -397,8 +417,9 @@ __device__ __forceinline__ void epi_batch(const ScanParams& p, const EpiCtx& c, 
   }
 }
 
-template <int PA, int PB, bool QC, bool RG>
-__device__ __forceinline__ void epi_tile(const ScanParams& p, const EpiCtx& c) {
+// release_acc: hands the tile's accumulators back to the MMA issuer; called as soon as the last batch is in registers.
+template <int PA, int PB, bool QC, bool RG, class Rel>
+__device__ __forceinline__ void epi_tile(const ScanParams& p, const EpiCtx& c, Rel&& release_acc) {
   constexpr int RA = PA + 1, RB = PB + 1;
   constexpr int JC = mi_jc(PA, PB);
   constexpr int NJ = 1 << mi_njlog2(PA, PB);
@@ -450,35 +471,38 @@ __device__ __forceinline__ void epi_tile(const ScanParams& p, const EpiCtx& c) {
 
   // ---- batches of JC columns, evaluated in lock step
   const int jbeg = c.cg * (NJ / MI_EPI_GROUPS);
-  uint32_t Ha[PA][PB][JC], La[PA][PB][JC];
+  uint32_t H[PA][PB][JC], L[PA][PB][JC];
 #pragma unroll 1
   for (int bi = 0; bi < NB; bi++) {
     const int j0 = jbeg + bi * JC;
-    epi_load<PA, PB, JC>(c.tmem_base, NJ, j0, Ha, La);
+    epi_load<PA, PB, JC>(c.tmem_base, NJ, j0, H, L);
     tmem_ld_wait();
-    epi_batch<PA, PB, JC, QC, RG>(p, c, k, j0, Ha, La);
+    if (bi + 1 == NB) release_acc();
+    uint32_t T[PA][PB][JC];
+    epi_counts<PA, PB, JC>(H, L, k.mul_a, k.sb, k.M, T);
+    epi_batch<PA, PB, JC, QC, RG>(p, c, k, j0, T);
   }
 }
 
-template <bool QC, bool RG>
-__device__ __forceinline__ void epi_dispatch(const ScanParams& p, int pa, int pb, const EpiCtx& c) {
+template <bool QC, bool RG, class Rel>
+__device__ __forceinline__ void epi_dispatch(const ScanParams& p, int pa, int pb, const EpiCtx& c, Rel&& rel) {
   switch (pa * 4 + pb - 5) {
-    case 0: epi_tile<1, 1, QC, RG>(p, c); break;
-    case 1: epi_tile<1, 2, QC, RG>(p, c); break;
-    case 2: epi_tile<1, 3, QC, RG>(p, c); break;
-    case 3: epi_tile<1, 4, QC, RG>(p, c); break;
-    case 4: epi_tile<2, 1, QC, RG>(p, c); break;
-    case 5: epi_tile<2, 2, QC, RG>(p, c); break;
-    case 6: epi_tile<2, 3, QC, RG>(p, c); break;
-    case 7: epi_tile<2, 4, QC, RG>(p, c); break;
-    case 8: epi_tile<3, 1, QC, RG>(p, c); break;
-    case 9: epi_tile<3, 2, QC, RG>(p, c); break;
-    case 10: epi_tile<3, 3, QC, RG>(p, c); break;
-    case 11: epi_tile<3, 4, QC, RG>(p, c); break;
-    case 12: epi_tile<4, 1, QC, RG>(p, c); break;
-    case 13: epi_tile<4, 2, QC, RG>(p, c); break;
-    case 14: epi_tile<4, 3, QC, RG>(p, c); break;
-    case 15: epi_tile<4, 4, QC, RG>(p, c); break;
+    case 0: epi_tile<1, 1, QC, RG>(p, c, rel); break;
+    case 1: epi_tile<1, 2, QC, RG>(p, c, rel); break;
+    case 2: epi_tile<1, 3, QC, RG>(p, c, rel); break;
+    case 3: epi_tile<1, 4, QC, RG>(p, c, rel); break;
+    case 4: epi_tile<2, 1, QC, RG>(p, c, rel); break;
+    case 5: epi_tile<2, 2, QC, RG>(p, c, rel); break;
+    case 6: epi_tile<2, 3, QC, RG>(p, c, rel); break;
+    case 7: epi_tile<2, 4, QC, RG>(p, c, rel); break;
+    case 8: epi_tile<3, 1, QC, RG>(p, c, rel); break;
+    case 9: epi_tile<3, 2, QC, RG>(p, c, rel); break;
+    case 10: epi_tile<3, 3, QC, RG>(p, c, rel); break;
+    case 11: epi_tile<3, 4, QC, RG>(p, c, rel); break;
+    case 12: epi_tile<4, 1, QC, RG>(p, c, rel); break;
+    case 13: epi_tile<4, 2, QC, RG>(p, c, rel); break;
+    case 14: epi_tile<4, 3, QC, RG>(p, c, rel); break;
+    case 15: epi_tile<4, 4, QC, RG>(p, c, rel); break;
     default: break;
   }
 }
@@ -785,21 +809,29 @@ mi_scan_kernel(const __grid_constant__ TmapSet tm, const __grid_constant__ ScanP
       }
       if constexpr (DBG) w_tfull += clock64() - c1;
       tc_fence_after();
+      // The accumulators belong to the pair: release them on the leader's barrier as soon as this warp holds the
+      // tile's last batch in registers (its tcgen05.wait::ld has returned; the fence orders the reads before the
+      // arrive), not after that batch's arithmetic -- the MMAs of the tile after next can start meanwhile.
+      bool released = false;
+      auto release_acc = [&]() {
+        tc_fence_before();
+        __syncwarp();
+        if (big) {
+          if (lane == 0) { mbar_arrive_cluster(&tempty[0], 0); mbar_arrive_cluster(&tempty[1], 0); }
+          aph ^= 1;  // two ring slots consumed: phase flips once
+        } else {
+          if (lane == 0) mbar_arrive_cluster(&tempty[as], 0);
+          if (++as == 2) { as = 0; aph ^= 1; }
+        }
+        released = true;
+      };
       if (!(c.tflags & TILE_NULL)) {
-        if (!p.qcorr) epi_dispatch<false, false>(p, tPA, tPB, c);
-        else if (p.ragged) epi_dispatch<true, true>(p, tPA, tPB, c);
-        else epi_dispatch<true, false>(p, tPA, tPB, c);
+        if (!p.qcorr) epi_dispatch<false, false>(p, tPA, tPB, c, release_acc);
+        else if (p.ragged) epi_dispatch<true, true>(p, tPA, tPB, c, release_acc);
+        else epi_dispatch<true, false>(p, tPA, tPB, c, release_acc);
       }
-      tc_fence_before();
+      if (!released) release_acc();
       __syncwarp();
-      // the accumulators belong to the pair: release them on the leader's barrier
-      if (big) {
-        if (lane == 0) { mbar_arrive_cluster(&tempty[0], 0); mbar_arrive_cluster(&tempty[1], 0); }
-        aph ^= 1;  // two ring slots consumed: phase flips once
-      } else {
-        if (lane == 0) mbar_arrive_cluster(&tempty[as], 0);
-        if (++as == 2) { as = 0; aph ^= 1; }
-      }
       if (lane == 0) mbar_arrive(&jempty[jb]);
     }
     if (DBG && p.dbg && lane == 0 && (warp == MI_EPI_WARP0 || warp == MI_EPI_WARP0 + MI_EPI_WARPS - 1)) {
