@@ -137,7 +137,8 @@ LDW_API int ldw_acgtn2num(ldw_ctx* ctx, double* nv, const char* ref, int64_t n);
  * ldw_hdw replaces the body of estimate_Hamming_distance_weights(snp.dat, threshold)
  *   (R/performPopulationStuctureCorrection.R:20-81; the five Matrix::crossprod calls :49-74 and
  *   the threshold/colSums/reciprocal :76).
- *   codes      : nsnp x nseq class matrix (== the five snp.matrix_* slots)
+ *   codes      : nsnp x nseq class matrix (== the five snp.matrix_* slots); a class outside 0..4 is refused with
+ *                LDW_ERR_ARG (checked on the device after the upload, as ldw_group_load_codes does)
  *   threshold  : fraction; thresh = (int)(nsnp*threshold) (truncation, :23)
  *   cnt_out    : nseq int32, #sequences (incl. self) with Hamming distance < thresh
  *   hdw_out    : nseq doubles, 1/(cnt+1)

@@ -264,6 +264,11 @@ int ldw_hdw(ldw_ctx* ctx, const uint8_t* codes, int64_t n_snp, int64_t nseq, dou
   LDW_TRY(d_w.alloc((size_t)nseq * 8));
   if (dist_out) LDW_TRY(d_dist.alloc((size_t)nseq * nseq * 4));
   LDW_CUDA(cudaMemcpyAsync(d_codes.p, codes, (size_t)n_snp * nseq, cudaMemcpyHostToDevice, st));
+  // every class must be 0..4 (as ldw_group_load_codes and ldw_mi_plan_create check): the plane packing compares a code
+  // with the allele index, so a byte above 4 would give distances that are neither the reference's nor an error
+  uint32_t mx = 0;
+  LDW_TRY(max_byte_device(st, d_codes.as<uint8_t>(), n_snp * nseq, &mx));
+  if (mx > 4) return set_error(LDW_ERR_ARG, "ldw_hdw: the matrix holds a class %u outside 0..4", mx);
   LDW_TRY(hdw_device(st, d_codes.as<uint8_t>(), n_snp, nseq, thresh, d_neigh.as<int32_t>(), d_w.as<double>(),
                      dist_out ? d_dist.as<int32_t>() : nullptr, ctx->num_sms));
   if (cnt_out) LDW_CUDA(cudaMemcpyAsync(cnt_out, d_neigh.p, (size_t)nseq * 4, cudaMemcpyDeviceToHost, st));

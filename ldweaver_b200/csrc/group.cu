@@ -264,13 +264,8 @@ int ldw_group_load_codes(ldw_group* G, const uint8_t* codes, int64_t n_snp, int6
     if (mb.rank == 0) {
       LDW_CUDA(cudaMemcpyAsync(mb.d_codes.p, codes, bytes, cudaMemcpyHostToDevice, st));
       // every class must be 0..4 (as ldw_mi_plan_create checks on the host): one pass at HBM speed on the device
-      DevBuf d_max;
-      LDW_TRY(d_max.alloc(4));
-      LDW_CUDA(cudaMemsetAsync(d_max.p, 0, 4, st));
-      LDW_TRY(max_byte_device(st, mb.d_codes.as<uint8_t>(), (int64_t)bytes, d_max.as<uint32_t>()));
       uint32_t mx = 0;
-      LDW_CUDA(cudaMemcpyAsync(&mx, d_max.p, 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaStreamSynchronize(st));
+      LDW_TRY(max_byte_device(st, mb.d_codes.as<uint8_t>(), (int64_t)bytes, &mx));
       if (mx > 4) bad_code = (int)mx;  // reported after the collective below, so that no rank is left waiting in it
     }
     if (G->world > 1) LDW_NCCL(nccl->Broadcast(mb.d_codes.p, mb.d_codes.p, bytes, ncclUint8, 0, mb.comm, st));

@@ -361,10 +361,16 @@ __global__ void max_byte_kernel(const uint8_t* __restrict__ p, int64_t n, uint32
   if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
 }
 
-int max_byte_device(cudaStream_t st, const uint8_t* d, int64_t n, uint32_t* d_out) {
+int max_byte_device(cudaStream_t st, const uint8_t* d, int64_t n, uint32_t* out) {
+  *out = 0;
   if (n <= 0) return 0;
-  max_byte_kernel<<<148 * 8, 256, 0, st>>>(d, n, d_out);
+  DevBuf d_max;
+  LDW_TRY(d_max.alloc(4));
+  LDW_CUDA(cudaMemsetAsync(d_max.p, 0, 4, st));
+  max_byte_kernel<<<148 * 8, 256, 0, st>>>(d, n, d_max.as<uint32_t>());
   LDW_CUDA(cudaGetLastError());
+  LDW_CUDA(cudaMemcpyAsync(out, d_max.p, 4, cudaMemcpyDeviceToHost, st));
+  LDW_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
 
