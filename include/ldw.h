@@ -156,6 +156,8 @@ LDW_API int ldw_hdw(ldw_ctx* ctx, const uint8_t* codes, int64_t n_snp, int64_t n
  *
  * ldw_mi_plan_create uploads one snp.dat (codes, uqe-derived allele sets, POS) and the weights, and
  * packs the tensor-core operands on the device.  `blk` is round(max_blk_sz, -3) (R/computePairwiseMI.R:69).
+ * A class outside 0..4 is refused with LDW_ERR_ARG (checked on the device after the upload, as
+ * ldw_group_load_codes does).
  */
 typedef struct ldw_links {
   int64_t n;             /* rows */

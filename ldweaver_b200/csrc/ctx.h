@@ -2,24 +2,40 @@
 #pragma once
 #include "host_util.h"
 
-// Link columns in pinned host memory (what ldw_links points into).  Owned by the context and reused by every
-// scan on it: allocating gigabytes of pinned memory costs far more than the scan itself.
-struct HostLinks {
-  ldw::PinnedBuf pos1, pos2, c1, c2, len, blk, mi;
+// The seven link columns pos1 pos2 c1 c2 len blk mi (int32 but mi, which is double) over one kind of buffer: pinned host
+// memory (HostLinks) or device memory (the scan's workspace).  col(k) and elem(k), k < NCOL, are column k and the
+// size of its element.
+template <class Buf>
+struct LinkCols {
+  static constexpr int NCOL = 7;
+  Buf pos1, pos2, c1, c2, len, blk, mi;
   int64_t n = 0;
+  static size_t elem(int k) { return k == 6 ? 8 : 4; }
+  Buf& col(int k) {
+    Buf* c[NCOL] = {&pos1, &pos2, &c1, &c2, &len, &blk, &mi};
+    return *c[k];
+  }
   int ensure(int64_t m) {
-    size_t b4 = (size_t)(m > 0 ? m : 1) * 4, b8 = (size_t)(m > 0 ? m : 1) * 8;
-    LDW_TRY(pos1.ensure(b4)); LDW_TRY(pos2.ensure(b4)); LDW_TRY(c1.ensure(b4)); LDW_TRY(c2.ensure(b4));
-    LDW_TRY(len.ensure(b4)); LDW_TRY(blk.ensure(b4)); LDW_TRY(mi.ensure(b8));
+    for (int k = 0; k < NCOL; k++) LDW_TRY(col(k).ensure((size_t)(m > 0 ? m : 1) * elem(k)));
     return 0;
   }
   void fill(ldw_links* o) const {
     if (!o) return;
     o->n = n;
-    o->pos1 = pos1.as<int32_t>(); o->pos2 = pos2.as<int32_t>(); o->clust1 = c1.as<int32_t>(); o->clust2 = c2.as<int32_t>();
-    o->len = len.as<int32_t>(); o->MI = mi.as<double>(); o->block = blk.as<int32_t>();
+    o->pos1 = pos1.template as<int32_t>(); o->pos2 = pos2.template as<int32_t>();
+    o->clust1 = c1.template as<int32_t>(); o->clust2 = c2.template as<int32_t>();
+    o->len = len.template as<int32_t>(); o->MI = mi.template as<double>(); o->block = blk.template as<int32_t>();
+  }
+  // column k of a table handed out through the ABI (the counterpart of fill)
+  static const char* abi_col(const ldw_links& L, int k) {
+    const void* c[NCOL] = {L.pos1, L.pos2, L.clust1, L.clust2, L.len, L.block, L.MI};
+    return static_cast<const char*>(c[k]);
   }
 };
+
+// Link columns in pinned host memory (what ldw_links points into).  Owned by the context and reused by every
+// scan on it: allocating gigabytes of pinned memory costs far more than the scan itself.
+using HostLinks = LinkCols<ldw::PinnedBuf>;
 
 struct ldw_ctx {
   int device = 0;

@@ -22,6 +22,7 @@
 
 #include <chrono>
 #include <cmath>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -263,7 +264,7 @@ int ldw_group_load_codes(ldw_group* G, const uint8_t* codes, int64_t n_snp, int6
     LDW_TRY(mb.d_codes.ensure(bytes));
     if (mb.rank == 0) {
       LDW_CUDA(cudaMemcpyAsync(mb.d_codes.p, codes, bytes, cudaMemcpyHostToDevice, st));
-      // every class must be 0..4 (as ldw_mi_plan_create checks on the host): one pass at HBM speed on the device
+      // every class must be 0..4 (as ldw_hdw and ldw_mi_plan_create check): one pass at HBM speed on the device
       uint32_t mx = 0;
       LDW_TRY(max_byte_device(st, mb.d_codes.as<uint8_t>(), (int64_t)bytes, &mx));
       if (mx > 4) bad_code = (int)mx;  // reported after the collective below, so that no rank is left waiting in it
@@ -328,34 +329,32 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
   return ldw::guarded("ldw_group_mi_scan", [&]() -> int {
     const int nl = (int)G->m.size();
     // ---- every member packs its operands from the resident matrix (no host -> device copy of the matrix here)
-    std::vector<ldw_mi_plan*> plans(nl, nullptr);
-    auto destroy_plans = [&]() {
-      for (int k = 0; k < nl; k++)
-        if (plans[k]) { ldw_mi_plan_destroy(plans[k]); plans[k] = nullptr; }
-    };
+    std::vector<std::unique_ptr<ldw_mi_plan, decltype(&ldw_mi_plan_destroy)>> plans;
+    for (int k = 0; k < nl; k++) plans.emplace_back(nullptr, ldw_mi_plan_destroy);
     const auto tp0 = std::chrono::steady_clock::now();
     int rc = for_members(G, [&](int k) -> int {
-      return mi_plan_create_impl(G->m[k].ctx, nullptr, G->m[k].d_codes.as<uint8_t>(), G->n_snp, G->nseq, hdw, pos, paint, blk, &plans[k]);
+      ldw_mi_plan* p = nullptr;
+      const int rk = mi_plan_create_impl(G->m[k].ctx, nullptr, G->m[k].d_codes.as<uint8_t>(), G->n_snp, G->nseq, hdw, pos,
+                                         paint, blk, &p);
+      plans[k].reset(p);
+      return rk;
     });
-    if (rc != 0) { destroy_plans(); return rc; }
+    if (rc != 0) return rc;
     if (t_plan_ms_out) *t_plan_ms_out = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp0).count();
     if (nl == 1) {  // one local member (a single device, or one rank of a multi-process job): exactly ldw_mi_scan over this rank's
                     // share -- its own sizing pass over its own blocks, its own tables, nothing to merge
       ldw_scan_stats st1;
-      rc = mi_scan_impl(plans[0], g, sr_dist, lr_retain_links, lr_links_approx, flags, G->world, G->m[0].rank, nullptr, sr_out, lr_out,
-                        borderline_out, thr_out, prob_out, &st1);
-      if (rc != 0) { std::string keep = last_error_ref(); destroy_plans(); return set_error(rc, "%s", keep.c_str()); }
-      destroy_plans();
+      LDW_TRY(mi_scan_impl(plans[0].get(), g, sr_dist, lr_retain_links, lr_links_approx, flags, G->world, G->m[0].rank, nullptr,
+                           sr_out, lr_out, borderline_out, thr_out, prob_out, &st1));
       if (stats_out) stats_out[0] = st1;
       return 0;
     }
     // ---- one layout for the job's short-range table: block sizes once, rows of the blocks this process scans
     ScanShared sh;
-    rc = mi_block_sizes(plans[0], g, sr_dist, flags, sh.sizes);
-    if (rc != 0) { destroy_plans(); return rc; }
-    const int64_t nblk = mi_plan_nblocks(plans[0]);
+    LDW_TRY(mi_block_sizes(plans[0].get(), g, sr_dist, flags, sh.sizes));
+    const int64_t nblk = mi_plan_nblocks(plans[0].get());
     std::vector<int> owner;
-    mi_block_owners(plans[0], G->world, owner);
+    mi_block_owners(plans[0].get(), G->world, owner);
     std::vector<char> local_rank(G->world, 0);
     for (auto& mb : G->m) local_rank[mb.rank] = 1;
     sh.sr_hbase.assign(nblk, 0);
@@ -370,19 +369,16 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
     G->h_sr.n = 0; G->h_lr.n = 0; G->h_border.n = 0;
     const bool sr_rows = !(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_LR_ONLY));
     if (!sr_rows) total_sr = 0;
-    if (want_host) {
-      rc = G->h_sr.ensure(total_sr);
-      if (rc != 0) { destroy_plans(); return rc; }
-    }
+    if (want_host) LDW_TRY(G->h_sr.ensure(total_sr));
     // ---- scan: one host thread per local device
     std::vector<ldw_links> lr(nl), bd(nl), srn(nl);
     std::vector<std::vector<double>> thr(nl, std::vector<double>(nblk, NAN)), prob(nl, std::vector<double>(nblk, NAN));
     std::vector<ldw_scan_stats> stats(nl);
     rc = for_members(G, [&](int k) -> int {
-      return mi_scan_impl(plans[k], g, sr_dist, lr_retain_links, lr_links_approx, flags, G->world, G->m[k].rank, &sh, &srn[k],
+      return mi_scan_impl(plans[k].get(), g, sr_dist, lr_retain_links, lr_links_approx, flags, G->world, G->m[k].rank, &sh, &srn[k],
                           &lr[k], &bd[k], thr[k].data(), prob[k].data(), &stats[k]);
     });
-    destroy_plans();
+    plans.clear();
     if (rc != 0) return rc;
     // ---- merge
     if (thr_out) for (int64_t b = 0; b < nblk; b++) thr_out[b] = NAN;
@@ -424,14 +420,10 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
       dst.n = total;
       int64_t o = 0;
       for (const Run& r : runs) {
-        const ldw_links& L = parts[r.k];
-        memcpy(dst.pos1.as<int32_t>() + o, L.pos1 + r.lo, (size_t)r.n * 4);
-        memcpy(dst.pos2.as<int32_t>() + o, L.pos2 + r.lo, (size_t)r.n * 4);
-        memcpy(dst.c1.as<int32_t>() + o, L.clust1 + r.lo, (size_t)r.n * 4);
-        memcpy(dst.c2.as<int32_t>() + o, L.clust2 + r.lo, (size_t)r.n * 4);
-        memcpy(dst.len.as<int32_t>() + o, L.len + r.lo, (size_t)r.n * 4);
-        memcpy(dst.blk.as<int32_t>() + o, L.block + r.lo, (size_t)r.n * 4);
-        memcpy(dst.mi.as<double>() + o, L.MI + r.lo, (size_t)r.n * 8);
+        for (int c = 0; c < HostLinks::NCOL; c++) {
+          const size_t e = HostLinks::elem(c);
+          memcpy(dst.col(c).as<char>() + o * e, HostLinks::abi_col(parts[r.k], c) + r.lo * e, (size_t)r.n * e);
+        }
         o += r.n;
       }
       return 0;

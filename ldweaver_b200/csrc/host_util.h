@@ -132,6 +132,34 @@ struct PinnedBuf {
   template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
+// Owning CUDA event.  Destroying it while recorded work is pending is allowed: the driver releases it on completion.
+struct Event {
+  cudaEvent_t e = nullptr;
+  Event() {}
+  Event(const Event&) = delete;
+  Event& operator=(const Event&) = delete;
+  Event(Event&& o) noexcept : e(o.e) { o.e = nullptr; }
+  Event& operator=(Event&& o) noexcept {
+    if (this != &o) {
+      release();
+      e = o.e;
+      o.e = nullptr;
+    }
+    return *this;
+  }
+  ~Event() { release(); }
+  void release() {
+    if (e) cudaEventDestroy(e);
+    e = nullptr;
+  }
+  int create(unsigned flags = cudaEventDefault) {
+    release();
+    LDW_CUDA(cudaEventCreateWithFlags(&e, flags));
+    return 0;
+  }
+  operator cudaEvent_t() const { return e; }
+};
+
 // 2-D uint8 tensor [rows][kbytes] (kbytes contiguous), box = 128 bytes x box_rows, 128B swizzle.
 int make_tmap_u8_sw128(CUtensorMap* out, const void* gptr, uint64_t rows, uint64_t kbytes, uint32_t box_rows);
 

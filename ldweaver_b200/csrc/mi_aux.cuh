@@ -240,30 +240,6 @@ __device__ __forceinline__ double refine_pair(const RefineParams& P, int il, int
   return mi;
 }
 
-// Candidates below the FINAL candidate threshold are an incomplete sample of their MI range (the threshold rose
-// while they were being collected); they cannot take part in the selection.  The others are refined to fp64 and
-// written compactly (vcand / vmi, count in *vcount).
-__global__ void mi_refine_cand_kernel(RefineParams P, const Cand* __restrict__ cand, const uint32_t* __restrict__ count,
-                                      uint32_t cap, const uint32_t* __restrict__ tcand_bits, int emit_all, Cand* vcand,
-                                      double* vmi, uint32_t* vcount) {
-  __shared__ double acc_s[REFINE_WARPS][32 * 25];
-  uint32_t n = *count < cap ? *count : cap;
-  const float tc = emit_all ? -3.0e38f : __uint_as_float(*tcand_bits);
-  int lane = threadIdx.x & 31;
-  double* acc = acc_s[threadIdx.x >> 5];
-  refine_scratch_clear(acc, threadIdx.x & 31);
-  for (uint32_t i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += gridDim.x * (blockDim.x >> 5)) {
-    Cand c = cand[i];
-    if (c.mi < tc) continue;
-    double v = refine_pair(P, c.il, c.jl, lane, acc);
-    if (lane == 0) {
-      uint32_t o = atomicAdd(vcount, 1u);
-      vcand[o] = c;
-      vmi[o] = v;
-    }
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // Pre-selection on the fp32 values the scan kernel produced.  The exact (fp64) K-th largest MI of a block lies within
 // eps (the fp32 epilogue's error, < 5e-7 measured) of the K-th largest fp32 value v32, and every candidate whose exact

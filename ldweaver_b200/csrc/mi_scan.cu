@@ -9,6 +9,7 @@
 #include <chrono>
 #include <cmath>
 #include <cub/cub.cuh>
+#include <memory>
 #include <vector>
 
 #include "../../include/ldw.h"
@@ -26,22 +27,14 @@ struct Group {
   int32_t slot0 = 0, nslots = 0, row0 = 0, count = 0;
 };
 
-struct DevLinks {
-  DevBuf pos1, pos2, c1, c2, len, blk, mi;
-  int ensure(int64_t m) {
-    size_t b4 = (size_t)(m > 0 ? m : 1) * 4, b8 = (size_t)(m > 0 ? m : 1) * 8;
-    LDW_TRY(pos1.ensure(b4)); LDW_TRY(pos2.ensure(b4)); LDW_TRY(c1.ensure(b4)); LDW_TRY(c2.ensure(b4));
-    LDW_TRY(len.ensure(b4)); LDW_TRY(blk.ensure(b4)); LDW_TRY(mi.ensure(b8));
-    return 0;
-  }
-};
+using DevLinks = LinkCols<DevBuf>;
 
 // Everything one block needs on the device besides the static plan.
 struct BlockDev {
   DevBuf rowdyn, coldyn, colinfo, tiles, from_idx, to_idx, rfl, rtl;
   PinnedBuf stage;
-  cudaEvent_t uploaded = nullptr;               // the block's tables have arrived (upload stream)
-  cudaEvent_t done = nullptr, done2 = nullptr;  // last use on the scan stream / on the select stream
+  Event uploaded;     // the block's tables have arrived (upload stream)
+  Event done, done2;  // last use on the scan stream / on the select stream
   bool used = false, used2 = false;
 };
 
@@ -70,7 +63,7 @@ struct ScanWS {
   // select stream while blocks b+1 and b+2 are being scanned into the other buffers
   struct LrBuf {
     DevBuf cand, vcand, mi64, state /*count, tcand, overflow, -, -, vcount*/, hist;
-    cudaEvent_t scan_done = nullptr, sel_done = nullptr;
+    Event scan_done, sel_done;
     bool used = false, chain_valid = false;
   } lr[3];
   static constexpr int NLR = 3;
@@ -80,17 +73,15 @@ struct ScanWS {
   PinnedBuf h_results, h_pub;
   DevBuf d_kept_key, d_kept_gi, d_kept_gj, d_kept_mi, d_kept_count, d_sort_tmp, d_keys_sorted, d_order_in, d_order_out;
   DevLinks d_sr, d_lr;
-  bool events_ready = false;
-  ~ScanWS() {
-    for (auto& b : ring) {
-      if (b.done) cudaEventDestroy(b.done);
-      if (b.done2) cudaEventDestroy(b.done2);
-      if (b.uploaded) cudaEventDestroy(b.uploaded);
-    }
-    for (auto& l : lr) {
-      if (l.scan_done) cudaEventDestroy(l.scan_done);
-      if (l.sel_done) cudaEventDestroy(l.sel_done);
-    }
+  // created by the first plan on the context (a failed creation is retried by the next)
+  int create_events() {
+    for (auto& b : ring)
+      for (Event* e : {&b.done, &b.done2, &b.uploaded})
+        if (!e->e) LDW_TRY(e->create(cudaEventDisableTiming));
+    for (auto& l : lr)
+      for (Event* e : {&l.scan_done, &l.sel_done})
+        if (!e->e) LDW_TRY(e->create(cudaEventDisableTiming));
+    return 0;
   }
 };
 
@@ -130,6 +121,20 @@ struct ldw_mi_plan {
 
 namespace {
 
+// One make_blocks block (R/computePairwiseMI.R:147-165): SNP ranges bf <= bt, and its row in the list.
+struct Blk {
+  int bf, bt;
+  int64_t index;
+};
+
+// The make_blocks list in its order (row-major over bf, bt >= bf): entry k has index k.
+std::vector<Blk> make_blocks(const ldw_mi_plan* P) {
+  std::vector<Blk> bl;
+  for (int i = 0; i < P->nranges; i++)
+    for (int j = i; j < P->nranges; j++) bl.push_back({i, j, (int64_t)bl.size()});
+  return bl;
+}
+
 // ---------------------------------------------------------------------------------------------- plan
 // codes: host class matrix (uploaded here), or NULL when `codes_dev` already holds it on this device (multi-GPU: the
 // group uploads once and broadcasts, ldw_group_load_codes)
@@ -138,9 +143,9 @@ int build_plan(ldw_mi_plan* P, const uint8_t* codes, const uint8_t* codes_dev, c
   ldw_ctx* ctx = P->ctx;
   cudaStream_t st = ctx->stream;
   const int64_t n = P->n, S = P->S, blk = P->blk;
-  cudaEvent_t e0, e1;
-  LDW_CUDA(cudaEventCreate(&e0));
-  LDW_CUDA(cudaEventCreate(&e1));
+  Event e0, e1;
+  LDW_TRY(e0.create());
+  LDW_TRY(e1.create());
   LDW_CUDA(cudaEventRecord(e0, st));
   const bool dbg_t = getenv("LDW_DBG_TIMING") != nullptr;
   auto bt0 = std::chrono::steady_clock::now();
@@ -258,7 +263,14 @@ int build_plan(ldw_mi_plan* P, const uint8_t* codes, const uint8_t* codes_dev, c
   LDW_TRY(P->d_r.alloc((size_t)n));
   DevBuf d_table;
   LDW_TRY(d_table.alloc((size_t)n * 5 * 4));
-  if (codes) LDW_CUDA(cudaMemcpyAsync(P->d_codes.p, codes, (size_t)n * S, cudaMemcpyHostToDevice, st));
+  if (codes) {
+    LDW_CUDA(cudaMemcpyAsync(P->d_codes.p, codes, (size_t)n * S, cudaMemcpyHostToDevice, st));
+    // every class must be 0..4 (the device group checked its matrix in ldw_group_load_codes): one pass at HBM speed,
+    // before any kernel reads the matrix
+    uint32_t mx = 0;
+    LDW_TRY(max_byte_device(st, P->codes_dev, n * S, &mx));
+    if (mx > 4) return set_error(LDW_ERR_ARG, "ldw_mi_plan_create: the matrix holds a class %u outside 0..4", mx);
+  }
   LDW_TRY(snp_allele_stats(st, P->codes_dev, n, S, d_table.as<int32_t>(), P->d_mask.as<uint8_t>(), P->d_r.as<uint8_t>()));
   P->r.resize(n);
   P->mask.resize(n);
@@ -357,29 +369,13 @@ int build_plan(ldw_mi_plan* P, const uint8_t* codes, const uint8_t* codes_dev, c
   uint64_t trows = (uint64_t)std::max<int64_t>(row, 128);
   LDW_TRY(make_tmap_u8_sw128(&P->tm.a, P->d_ops.p, trows, (uint64_t)P->Kpad, 128));
   for (int j = 0; j < 4; j++) LDW_TRY(make_tmap_u8_sw128(&P->tm.b[j], P->d_ops.p, trows, (uint64_t)P->Kpad, 64u >> j));
-  {
-    ScanWS* W = get_ws(ctx);
-    if (!W->events_ready) {
-      for (auto& b : W->ring) {
-        LDW_CUDA(cudaEventCreateWithFlags(&b.done, cudaEventDisableTiming));
-        LDW_CUDA(cudaEventCreateWithFlags(&b.done2, cudaEventDisableTiming));
-        LDW_CUDA(cudaEventCreateWithFlags(&b.uploaded, cudaEventDisableTiming));
-      }
-      for (auto& l : W->lr) {
-        LDW_CUDA(cudaEventCreateWithFlags(&l.scan_done, cudaEventDisableTiming));
-        LDW_CUDA(cudaEventCreateWithFlags(&l.sel_done, cudaEventDisableTiming));
-      }
-      W->events_ready = true;
-    }
-  }
+  LDW_TRY(get_ws(ctx)->create_events());
   LDW_CUDA(cudaEventRecord(e1, st));
   LDW_CUDA(cudaStreamSynchronize(st));
   blap("records + pack + tmaps");
   float ms = 0;
   cudaEventElapsedTime(&ms, e0, e1);
   P->t_pack_ms = ms;
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
   LDW_CUDA(cudaFuncSetAttribute(mi_scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MI_SMEM_BYTES));
   LDW_CUDA(cudaFuncSetAttribute(mi_scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MI_SMEM_BYTES));
   return 0;
@@ -387,7 +383,7 @@ int build_plan(ldw_mi_plan* P, const uint8_t* codes, const uint8_t* codes_dev, c
 
 // ---------------------------------------------------------------------------------------------- per-block host prep
 struct ScanCfg {
-  double g, sr_dist, lr_retain, lr_approx;
+  double g, sr_dist;
   int flags;
   int dense = 0;  // debug: every (row, col) cell is wanted, so no tile is skipped
 };
@@ -743,7 +739,9 @@ extern "C" {
 int ldw_mi_plan_create(ldw_ctx* ctx, const uint8_t* codes, int64_t n_snp, int64_t nseq, const double* hdw,
                        const int32_t* pos, const int32_t* paint, int64_t blk, ldw_mi_plan** out) {
   if (!codes) return set_error(LDW_ERR_ARG, "ldw_mi_plan_create: null argument");
-  return ldw::mi_plan_create_impl(ctx, codes, nullptr, n_snp, nseq, hdw, pos, paint, blk, out);
+  return ldw::guarded("ldw_mi_plan_create", [&]() -> int {
+    return ldw::mi_plan_create_impl(ctx, codes, nullptr, n_snp, nseq, hdw, pos, paint, blk, out);
+  });
 }
 
 }  // extern "C"
@@ -757,34 +755,19 @@ int ldw::mi_plan_create_impl(ldw_ctx* ctx, const uint8_t* codes, const uint8_t* 
   if (n_snp < 2 || nseq < 1) return set_error(LDW_ERR_ARG, "ldw_mi_plan_create: need at least 2 SNPs and 1 sequence");
   if (nseq > 65535) return set_error(LDW_ERR_UNSUPPORTED, "ldw_mi_plan_create: nseq > 65535 not supported by the 15-bit digit accumulation");
   if (blk < 128 || blk > 65535) return set_error(LDW_ERR_UNSUPPORTED, "ldw_mi_plan_create: block size %lld outside [128, 65535]", (long long)blk);
-  if (codes) {
-    // every code must be 0..4; eight bytes per step (a byte > 4 sets bit 7 of byte + 0x7B, or has it set already),
-    // chunks spread over a few host threads
-    const int64_t total = n_snp * nseq;
-    const int64_t chunk = (int64_t)1 << 22;
-    const int64_t nchunks = (total + chunk - 1) / chunk;
-    std::vector<int64_t> bad_at(nchunks, -1);
-    parallel_for(nchunks, 8, [&](int64_t c) {
-      int64_t i = c * chunk;
-      const int64_t end = std::min<int64_t>(total, i + chunk);
-      for (; i + 8 <= end; i += 8) {
-        uint64_t x;
-        memcpy(&x, codes + i, 8);
-        if ((((x & 0x7F7F7F7F7F7F7F7Full) + 0x7B7B7B7B7B7B7B7Bull) | x) & 0x8080808080808080ull) break;
-      }
-      for (; i < end; i++)
-        if (codes[i] > 4) { bad_at[c] = i; break; }
-    });
-    for (int64_t c = 0; c < nchunks; c++)
-      if (bad_at[c] >= 0)
-        return set_error(LDW_ERR_ARG, "ldw_mi_plan_create: codes[%lld] = %d outside 0..4", (long long)bad_at[c], (int)codes[bad_at[c]]);
-  }
-  ldw_mi_plan* P = new ldw_mi_plan();
+  std::unique_ptr<ldw_mi_plan> P(new ldw_mi_plan());
   P->ctx = ctx;
   P->n = n_snp; P->S = nseq; P->blk = blk;
-  int rc = build_plan(P, codes, codes_dev, hdw, pos, paint);
-  if (rc != 0) { delete P; return rc; }
-  *out = P;
+  LDW_TRY(build_plan(P.get(), codes, codes_dev, hdw, pos, paint));
+  *out = P.release();
+  return 0;
+}
+
+// Block `block_index` of the make_blocks list.
+static int block_at(const ldw_mi_plan* P, int64_t block_index, Blk* out) {
+  const std::vector<Blk> bl = make_blocks(P);
+  if (block_index < 0 || block_index >= (int64_t)bl.size()) return set_error(LDW_ERR_ARG, "block index out of range");
+  *out = bl[block_index];
   return 0;
 }
 
@@ -798,94 +781,81 @@ void ldw_mi_plan_destroy(ldw_mi_plan* plan) {
 
 int ldw_mi_block_dense(ldw_mi_plan* P, int64_t block_index, double* mi_out, int64_t* nf_out, int64_t* nt_out) {
   if (!P) return set_error(LDW_ERR_ARG, "null plan");
-  LDW_TRY(ctx_bind(P->ctx));
-  cudaStream_t st = P->ctx->stream;
-  ScanWS* W = get_ws(P->ctx);
-  // block_index -> (bf, bt) in make_blocks order
-  int bf = 0, bt = 0;
-  {
-    int64_t k = block_index;
-    bool found = false;
-    for (int i = 0; i < P->nranges && !found; i++)
-      for (int j = i; j < P->nranges; j++) {
-        if (k == 0) { bf = i; bt = j; found = true; break; }
-        k--;
-      }
-    if (!found) return set_error(LDW_ERR_ARG, "block index out of range");
-  }
-  ScanCfg cfg{1e15, 0.0, 0, 0, 0};
-  cfg.dense = 1;
-  BlockHost& H = W->hring[0];
-  BlockDev& D = W->ring[0];
-  int e = prepare_block(P, bf, bt, cfg, H);
-  if (e > 1) return e;
-  if (nf_out) *nf_out = H.nf;
-  if (nt_out) *nt_out = H.nt;
-  if (!mi_out) return 0;
-  LDW_TRY(upload_block(st, D, H));
-  size_t cells = (size_t)H.nf * H.nt;
-  LDW_TRY(W->d_dense.ensure(cells * 4));
-  LDW_CUDA(cudaMemsetAsync(W->d_dense.p, 0, cells * 4, st));
-  ScanParams sp;
-  fill_scan_params(P, D, H, cfg, sp);
-  sp.dense = 1;
-  sp.dense_out = W->d_dense.as<float>();
-  LDW_TRY(launch_scan(P, sp, st));
-  DevBuf d64;
-  LDW_TRY(d64.alloc(cells * 8));
-  f32_to_f64_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(W->d_dense.as<float>(), (int64_t)cells, d64.as<double>());
-  LDW_CUDA(cudaMemcpyAsync(mi_out, d64.p, cells * 8, cudaMemcpyDeviceToHost, st));
-  LDW_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return ldw::guarded("ldw_mi_block_dense", [&]() -> int {
+    LDW_TRY(ctx_bind(P->ctx));
+    cudaStream_t st = P->ctx->stream;
+    ScanWS* W = get_ws(P->ctx);
+    Blk k{};
+    LDW_TRY(block_at(P, block_index, &k));
+    ScanCfg cfg{1e15, 0.0, 0};
+    cfg.dense = 1;
+    BlockHost& H = W->hring[0];
+    BlockDev& D = W->ring[0];
+    int e = prepare_block(P, k.bf, k.bt, cfg, H);
+    if (e > 1) return e;
+    if (nf_out) *nf_out = H.nf;
+    if (nt_out) *nt_out = H.nt;
+    if (!mi_out) return 0;
+    LDW_TRY(upload_block(st, D, H));
+    size_t cells = (size_t)H.nf * H.nt;
+    LDW_TRY(W->d_dense.ensure(cells * 4));
+    LDW_CUDA(cudaMemsetAsync(W->d_dense.p, 0, cells * 4, st));
+    ScanParams sp;
+    fill_scan_params(P, D, H, cfg, sp);
+    sp.dense = 1;
+    sp.dense_out = W->d_dense.as<float>();
+    LDW_TRY(launch_scan(P, sp, st));
+    DevBuf d64;
+    LDW_TRY(d64.alloc(cells * 8));
+    f32_to_f64_kernel<<<(unsigned)((cells + 255) / 256), 256, 0, st>>>(W->d_dense.as<float>(), (int64_t)cells, d64.as<double>());
+    LDW_CUDA(cudaMemcpyAsync(mi_out, d64.p, cells * 8, cudaMemcpyDeviceToHost, st));
+    LDW_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  });
 }
 
 int ldw_mi_pairs_exact(ldw_mi_plan* P, int64_t block_index, const int32_t* from_local, const int32_t* to_local,
                        int64_t n_pairs, double* mi_out) {
   if (!P) return set_error(LDW_ERR_ARG, "null plan");
-  LDW_TRY(ctx_bind(P->ctx));
-  cudaStream_t st = P->ctx->stream;
-  ScanWS* W = get_ws(P->ctx);
-  int bf = 0, bt = 0;
-  {
-    int64_t k = block_index;
-    bool found = false;
-    for (int i = 0; i < P->nranges && !found; i++)
-      for (int j = i; j < P->nranges; j++) {
-        if (k == 0) { bf = i; bt = j; found = true; break; }
-        k--;
-      }
-    if (!found) return set_error(LDW_ERR_ARG, "block index out of range");
-  }
-  if (n_pairs <= 0) return 0;
-  ScanCfg cfg{1e15, 0.0, 0, 0, 0};
-  BlockHost& H = W->hring[0];
-  BlockDev& D = W->ring[0];
-  int e = prepare_block(P, bf, bt, cfg, H);
-  if (e != 0) return e == 1 ? set_error(LDW_ERR_ARG, "empty block") : e;
-  for (int64_t k = 0; k < n_pairs; k++)
-    if (from_local[k] < 0 || from_local[k] >= H.nf || to_local[k] < 0 || to_local[k] >= H.nt)
-      return set_error(LDW_ERR_ARG, "pair %lld outside the block", (long long)k);
-  LDW_TRY(upload_block(st, D, H));
-  DevBuf di, dj, dout;
-  LDW_TRY(di.alloc((size_t)n_pairs * 4));
-  LDW_TRY(dj.alloc((size_t)n_pairs * 4));
-  LDW_TRY(dout.alloc((size_t)n_pairs * 8));
-  LDW_CUDA(cudaMemcpyAsync(di.p, from_local, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, st));
-  LDW_CUDA(cudaMemcpyAsync(dj.p, to_local, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, st));
-  RefineParams R = make_refine_params(P, D, H, cfg);
-  int grid = (int)std::min<int64_t>((n_pairs + REFINE_WARPS - 1) / REFINE_WARPS, 148 * 8);
-  mi_refine_pairs_kernel<<<grid, 32 * REFINE_WARPS, 0, st>>>(R, di.as<int32_t>(), dj.as<int32_t>(), n_pairs, dout.as<double>());
-  LDW_CUDA(cudaGetLastError());
-  LDW_CUDA(cudaMemcpyAsync(mi_out, dout.p, (size_t)n_pairs * 8, cudaMemcpyDeviceToHost, st));
-  LDW_CUDA(cudaStreamSynchronize(st));
-  return 0;
+  return ldw::guarded("ldw_mi_pairs_exact", [&]() -> int {
+    LDW_TRY(ctx_bind(P->ctx));
+    cudaStream_t st = P->ctx->stream;
+    ScanWS* W = get_ws(P->ctx);
+    Blk k{};
+    LDW_TRY(block_at(P, block_index, &k));
+    if (n_pairs <= 0) return 0;
+    ScanCfg cfg{1e15, 0.0, 0};
+    BlockHost& H = W->hring[0];
+    BlockDev& D = W->ring[0];
+    int e = prepare_block(P, k.bf, k.bt, cfg, H);
+    if (e != 0) return e == 1 ? set_error(LDW_ERR_ARG, "empty block") : e;
+    for (int64_t i = 0; i < n_pairs; i++)
+      if (from_local[i] < 0 || from_local[i] >= H.nf || to_local[i] < 0 || to_local[i] >= H.nt)
+        return set_error(LDW_ERR_ARG, "pair %lld outside the block", (long long)i);
+    LDW_TRY(upload_block(st, D, H));
+    DevBuf di, dj, dout;
+    LDW_TRY(di.alloc((size_t)n_pairs * 4));
+    LDW_TRY(dj.alloc((size_t)n_pairs * 4));
+    LDW_TRY(dout.alloc((size_t)n_pairs * 8));
+    LDW_CUDA(cudaMemcpyAsync(di.p, from_local, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, st));
+    LDW_CUDA(cudaMemcpyAsync(dj.p, to_local, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, st));
+    RefineParams R = make_refine_params(P, D, H, cfg);
+    int grid = (int)std::min<int64_t>((n_pairs + REFINE_WARPS - 1) / REFINE_WARPS, 148 * 8);
+    mi_refine_pairs_kernel<<<grid, 32 * REFINE_WARPS, 0, st>>>(R, di.as<int32_t>(), dj.as<int32_t>(), n_pairs, dout.as<double>());
+    LDW_CUDA(cudaGetLastError());
+    LDW_CUDA(cudaMemcpyAsync(mi_out, dout.p, (size_t)n_pairs * 8, cudaMemcpyDeviceToHost, st));
+    LDW_CUDA(cudaStreamSynchronize(st));
+    return 0;
+  });
 }
 
 int ldw_mi_scan(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links, double lr_links_approx, int flags,
                 int n_parts, int part, ldw_links* sr_out, ldw_links* lr_out, ldw_links* borderline_out, double* thr_out,
                 double* prob_out, ldw_scan_stats* stats_out) {
-  return ldw::mi_scan_impl(P, g, sr_dist, lr_retain_links, lr_links_approx, flags, n_parts, part, nullptr, sr_out, lr_out,
-                           borderline_out, thr_out, prob_out, stats_out);
+  return ldw::guarded("ldw_mi_scan", [&]() -> int {
+    return ldw::mi_scan_impl(P, g, sr_dist, lr_retain_links, lr_links_approx, flags, n_parts, part, nullptr, sr_out, lr_out,
+                             borderline_out, thr_out, prob_out, stats_out);
+  });
 }
 
 }  // extern "C"
@@ -893,21 +863,19 @@ int ldw_mi_scan(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links
 // Sizes of every make_blocks block (pairs, short-range, long-range) on host threads: positions only, no device work.
 int ldw::mi_block_sizes(const ldw_mi_plan* P, double g, double sr_dist, int flags, std::vector<BlockSizes>& out) {
   if (!P) return set_error(LDW_ERR_ARG, "null plan");
-  ScanCfg cfg{g, sr_dist, 0, 0, flags};
+  ScanCfg cfg{g, sr_dist, flags};
   LDW_TRY(validate_scan(P, cfg));
-  std::vector<std::pair<int, int>> bl;
-  for (int i = 0; i < P->nranges; i++)
-    for (int j = i; j < P->nranges; j++) bl.push_back({i, j});
+  const std::vector<Blk> bl = make_blocks(P);
   out.assign(bl.size(), BlockSizes{0, 0, 0, 0});
   parallel_for((int64_t)bl.size(), 16, [&](int64_t b) {
     BlockHost tmp;
-    int e = prepare_block(P, bl[b].first, bl[b].second, cfg, tmp, true);
+    int e = prepare_block(P, bl[b].bf, bl[b].bt, cfg, tmp, true);
     out[b] = BlockSizes{tmp.n_pairs, tmp.n_sr, tmp.n_lr, e};
   });
   for (size_t b = 0; b < bl.size(); b++)
     if (out[b].err > 1) {  // re-run on this thread so that the (thread-local) error message is the caller's
       BlockHost t2;
-      return prepare_block(P, bl[b].first, bl[b].second, cfg, t2, true);
+      return prepare_block(P, bl[b].bf, bl[b].bt, cfg, t2, true);
     }
   return 0;
 }
@@ -918,13 +886,11 @@ int ldw::mi_block_sizes(const ldw_mi_plan* P, double g, double sr_dist, int flag
 void ldw::mi_block_owners(const ldw_mi_plan* P, int n_parts, std::vector<int>& owner) {
   struct Item { int64_t cost, idx; };
   std::vector<Item> items;
-  int64_t idx = 0;
-  for (int i = 0; i < P->nranges; i++)
-    for (int j = i; j < P->nranges; j++, idx++) {
-      const int64_t ni = std::min<int64_t>(P->n, (int64_t)(i + 1) * P->blk) - (int64_t)i * P->blk;
-      const int64_t nj = std::min<int64_t>(P->n, (int64_t)(j + 1) * P->blk) - (int64_t)j * P->blk;
-      items.push_back({i == j ? ni * (ni - 1) / 2 : ni * nj, idx});
-    }
+  auto rows = [P](int r) { return std::min<int64_t>(P->n, (int64_t)(r + 1) * P->blk) - (int64_t)r * P->blk; };
+  for (const Blk& k : make_blocks(P)) {
+    const int64_t ni = rows(k.bf), nj = rows(k.bt);
+    items.push_back({k.bf == k.bt ? ni * (ni - 1) / 2 : ni * nj, k.index});
+  }
   std::vector<Item> order = items;
   std::stable_sort(order.begin(), order.end(), [](const Item& a, const Item& b) { return a.cost > b.cost; });
   std::vector<int64_t> load(n_parts, 0);
@@ -938,51 +904,120 @@ void ldw::mi_block_owners(const ldw_mi_plan* P, int n_parts, std::vector<int>& o
   }
 }
 
-int64_t ldw::mi_plan_nblocks(const ldw_mi_plan* P) { return (int64_t)P->nranges * (P->nranges + 1) / 2; }
+int64_t ldw::mi_plan_nblocks(const ldw_mi_plan* P) { return (int64_t)make_blocks(P).size(); }
 
-int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links, double lr_links_approx, int flags,
-                      int n_parts, int part, const ScanShared* shared, ldw_links* sr_out, ldw_links* lr_out,
-                      ldw_links* borderline_out, double* thr_out, double* prob_out, ldw_scan_stats* stats_out) {
-  if (!P) return set_error(LDW_ERR_ARG, "null plan");
-  const auto t_entry = std::chrono::steady_clock::now();
-  LDW_TRY(ctx_bind(P->ctx));
-  cudaStream_t st = P->ctx->stream;
-  ScanWS* W = get_ws(P->ctx);
-  ScanCfg cfg{g, sr_dist, lr_retain_links, lr_links_approx, flags};
-  LDW_TRY(validate_scan(P, cfg));
-  const bool sr_only = (flags & LDW_SCAN_SR_ONLY) != 0;
-  if (!sr_only && !(lr_links_approx > 0)) return set_error(LDW_ERR_ARG, "lr_links_approx must be > 0");
-  if (n_parts < 1 || part < 0 || part >= n_parts) return set_error(LDW_ERR_ARG, "bad partition %d of %d", part, n_parts);
+namespace {
 
-  // ---- block list (make_blocks order), this part's share.  Blocks are dealt by cost (pairs), largest first, each to
-  //      the least-loaded part (lowest part on ties): diagonal blocks cost half of the others, so plain round-robin
-  //      would leave up to 12 % imbalance at 8 parts.  Deterministic: every rank derives the same assignment.
-  struct Blk { int bf, bt; int64_t index; };
-  std::vector<Blk> blocks;
-  {
+// ---------------------------------------------------------------------------------------------- the scan
+// One block of a scan: its sizes, its output offsets and the long-range selection (type-7 ranks, candidate buffer).
+struct Sel { int64_t n_lr = 0, n_sr = 0, n_pairs = 0; double prob = NAN; uint64_t k_lo = 0, k_hi = 0; double h = 0; int interp = 0;
+             int emit_all = 0; uint32_t kprime = 0, delta = 1, cap = 0; int64_t sr_base = 0, sr_hbase = 0; int skip = 0; };
+
+// How run_block collects a block's long-range candidates.  The first pass starts from the threshold the earlier blocks
+// left; a re-run starts from zero, and the last one collects every long-range pair into a buffer of `cap_override`.
+struct Attempt {
+  bool force_emit_all;
+  uint32_t cap_override;  // 0: the block's own cap
+  bool use_chain;
+  double sel_margin;
+};
+
+// Points a scan launch's long-range candidate collection at buffer L (the pilot launch and the main launch).
+void arm_collection(ScanParams& sp, const ScanWS::LrBuf& L, const Sel& s, uint32_t cap, int emit_all) {
+  uint32_t* d_count = L.state.as<uint32_t>();
+  sp.cand = L.cand.as<Cand>(); sp.cand_cap = cap; sp.cand_count = d_count; sp.tcand_bits = d_count + 1;
+  sp.hist = L.hist.as<uint32_t>(); sp.kprime = s.kprime; sp.delta = s.delta ? s.delta : 1; sp.overflow = d_count + 2;
+  sp.emit_all = emit_all;
+}
+
+// One call of mi_scan_impl: what its phases share.  mi_scan_impl runs the phases in order; the events are released on
+// every return.
+struct ScanRun {
+  using clock = std::chrono::steady_clock;
+  ldw_mi_plan* P;
+  ScanWS* W;
+  const ScanCfg cfg;
+  const double lr_retain_links, lr_links_approx;
+  const ScanShared* shared;
+  const int n_parts;
+  const bool sr_only;
+  const bool sr_rows;     // short-range link columns wanted at all
+  const bool sr_to_host;  // short-range rows cross PCIe at all?
+  cudaStream_t st, sst, cst;  // scan, select and copy streams
+  // short-range rows go to this context's pinned table, or -- multi-GPU -- straight to the group's table, every rank
+  // at the final offsets of its blocks (the table is complete when the last rank finishes: no merge pass)
+  HostLinks& hsr;
+
+  // test hooks and tuning
+  int64_t dbg_block = -1;
+  int scan_reserve = 2;  // SMs left to the selection stream (presel, refine, select of earlier blocks); 1-3 within 1 % at C2
+  // force every block's first attempt to start from this candidate threshold (a value above the true threshold makes
+  // the selection fail its completeness check and exercises the re-run path)
+  float force_seed = -1.f;
+  // margin of the long-range selection (pre-selection window and completeness test): sound while twice the fp32
+  // epilogue's error stays below it; the selection kernel measures that error per block and asks for a re-run with a
+  // wider margin when it does not (BlockResult.bad & 8)
+  double sel_margin0 = 4e-6;
+  const bool dbg_timing = getenv("LDW_DBG_TIMING") != nullptr;
+  const clock::time_point t_entry;
+  clock::time_point tpre, tp0;
+
+  int64_t nblk_total = 0;
+  std::vector<Blk> blocks;  // this part's share of make_blocks (b: index into it)
+  std::vector<Sel> sel;     // per entry of `blocks`
+  int64_t total_sr = 0, total_pairs = 0, total_lr = 0;
+  uint64_t max_cap = 1, sum_keep = 0, kept_cap = 0;
+  int64_t first_guess = -1;  // entry of `blocks` whose tables pass 1 builds into ring slot 0 ...
+  int first_rc = -1;         // ... and what prepare_block returned for it
+  uint32_t* d_chain = nullptr;
+  unsigned long long n_kept = 0;
+  int64_t n_reruns = 0, n_launches = 0, n_scan_launches = 0, n_tiles = 0;
+  double exec_ops = 0, exec_mufu = 0, host_prep_ms = 0;
+  Event ev0, ev1, ev2, ev3;  // around the scan, the long-range sort and the device -> host copies
+  Event ev_blk;              // "this block's SR columns are materialised"
+  std::vector<Event> kev;    // pairs of events around every scan-kernel launch
+
+  ScanRun(ldw_mi_plan* P_, const ScanCfg& cfg_, double retain, double approx, int n_parts_, const ScanShared* shared_,
+          clock::time_point t_entry_)
+      : P(P_), W(get_ws(P_->ctx)), cfg(cfg_), lr_retain_links(retain), lr_links_approx(approx), shared(shared_),
+        n_parts(n_parts_), sr_only((cfg_.flags & LDW_SCAN_SR_ONLY) != 0),
+        sr_rows(!(cfg_.flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_LR_ONLY))),
+        sr_to_host(!(cfg_.flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H | LDW_SCAN_SR_ON_DEVICE))),
+        st(P_->ctx->stream), sst(P_->ctx->select_stream), cst(P_->ctx->copy_stream),
+        hsr(shared_ ? *shared_->h_sr : P_->ctx->h_sr), t_entry(t_entry_) {
+    if (const char* e = getenv("LDW_DBG_BLOCK")) dbg_block = atoll(e);
+    if (const char* e = getenv("LDW_SCAN_RESERVE")) scan_reserve = atoi(e);
+    if (const char* e = getenv("LDW_DBG_FORCE_SEED")) force_seed = (float)atof(e);
+    if (const char* e = getenv("LDW_DBG_SEL_MARGIN")) sel_margin0 = atof(e);  // a tiny margin exercises that re-run
+  }
+
+  void lap(const char* what) {
+    if (!dbg_timing) return;
+    cudaStreamSynchronize(st);
+    auto t = clock::now();
+    fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(t - tp0).count());
+    tp0 = t;
+  }
+
+  // Checks the call and takes this part's share of the block list.
+  int take_share(int part, double* thr_out, double* prob_out) {
+    LDW_TRY(validate_scan(P, cfg));
+    if (!sr_only && !(lr_links_approx > 0)) return set_error(LDW_ERR_ARG, "lr_links_approx must be > 0");
+    if (n_parts < 1 || part < 0 || part >= n_parts) return set_error(LDW_ERR_ARG, "bad partition %d of %d", part, n_parts);
     std::vector<int> owner;
     mi_block_owners(P, n_parts, owner);
-    int64_t idx = 0;
-    for (int i = 0; i < P->nranges; i++)
-      for (int j = i; j < P->nranges; j++, idx++)
-        if (owner[idx] == part) blocks.push_back({i, j, idx});
+    for (const Blk& k : make_blocks(P))
+      if (owner[k.index] == part) blocks.push_back(k);
+    nblk_total = (int64_t)owner.size();
+    if (thr_out) for (int64_t b = 0; b < nblk_total; b++) thr_out[b] = NAN;
+    if (prob_out) for (int64_t b = 0; b < nblk_total; b++) prob_out[b] = NAN;
+    LDW_TRY(ev0.create()); LDW_TRY(ev1.create()); LDW_TRY(ev2.create()); LDW_TRY(ev3.create());
+    return 0;
   }
-  const int64_t nblk_total = (int64_t)P->nranges * (P->nranges + 1) / 2;
-  if (thr_out) for (int64_t b = 0; b < nblk_total; b++) thr_out[b] = NAN;
-  if (prob_out) for (int64_t b = 0; b < nblk_total; b++) prob_out[b] = NAN;
 
-  cudaEvent_t ev0, ev1, ev2, ev3;
-  LDW_CUDA(cudaEventCreate(&ev0)); LDW_CUDA(cudaEventCreate(&ev1)); LDW_CUDA(cudaEventCreate(&ev2)); LDW_CUDA(cudaEventCreate(&ev3));
-
-  // ---- pass 1 (host): per-block sizes -> output offsets and long-range selection ranks
-  struct Sel { int64_t n_lr = 0, n_sr = 0, n_pairs = 0; double prob = NAN; uint64_t k_lo = 0, k_hi = 0; double h = 0; int interp = 0;
-               int emit_all = 0; uint32_t kprime = 0, delta = 1, cap = 0; int64_t sr_base = 0, sr_hbase = 0; int skip = 0; };
-  std::vector<Sel> sel(blocks.size());
-  int64_t total_sr = 0, total_pairs = 0, total_lr = 0;
-  uint64_t max_cap = 1, sum_keep = 0;
-  int64_t first_guess = -1;
-  int first_rc = -1;
-  {
+  // Pass 1 (host): per-block sizes -> output offsets and long-range selection ranks.
+  int size_blocks() {
+    sel.resize(blocks.size());
     // block sizes on a few host threads (they gate the first launch), then the serial prefix / rank arithmetic
     std::vector<int> perr(blocks.size(), 0);
     // The block that will run first (the first one holding short-range links: diagonal or next to it) gets its full
@@ -1015,32 +1050,31 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
       }
       Sel& s = sel[b];
       s.skip = (e == 1);
-      struct { int64_t n_lr, n_sr, n_pairs; } tmp{s.n_lr, s.n_sr, s.n_pairs};
       s.sr_base = total_sr;
       s.sr_hbase = shared ? shared->sr_hbase[blocks[b].index] : total_sr;  // row of the block in the host table
-      total_sr += tmp.n_sr; total_pairs += tmp.n_pairs; total_lr += tmp.n_lr;
-      if (!sr_only && tmp.n_lr > 0) {
-        const double m = (double)tmp.n_lr;
+      total_sr += s.n_sr; total_pairs += s.n_pairs; total_lr += s.n_lr;
+      if (!sr_only && s.n_lr > 0) {
+        const double m = (double)s.n_lr;
         double prob = 1 - ((lr_retain_links * (m / lr_links_approx)) / m);  // R/computePairwiseMI.R:352
         if (prob < 0) prob = 0;
         s.prob = prob;
         double index = 1 + (m - 1 > 0 ? m - 1 : 0) * prob;  // stats::quantile type 7
         double lo = std::floor(index), hi = std::ceil(index);
-        s.k_lo = (uint64_t)(tmp.n_lr - (int64_t)lo + 1);
-        s.k_hi = (uint64_t)(tmp.n_lr - (int64_t)hi + 1);
+        s.k_lo = (uint64_t)(s.n_lr - (int64_t)lo + 1);
+        s.k_hi = (uint64_t)(s.n_lr - (int64_t)hi + 1);
         s.h = index - lo;
         s.interp = index > lo;
         uint64_t K = s.k_lo;
-        if (2 * K + 65536 >= (uint64_t)tmp.n_lr) {
+        if (2 * K + 65536 >= (uint64_t)s.n_lr) {
           s.emit_all = 1;
-          if ((uint64_t)tmp.n_lr > 0xFFFFFFF0ull) return set_error(LDW_ERR_UNSUPPORTED, "block keeps more than 2^32 long-range links");
-          s.cap = (uint32_t)tmp.n_lr;
+          if ((uint64_t)s.n_lr > 0xFFFFFFF0ull) return set_error(LDW_ERR_UNSUPPORTED, "block keeps more than 2^32 long-range links");
+          s.cap = (uint32_t)s.n_lr;
           s.kprime = (uint32_t)std::min<uint64_t>(K, 0xFFFFFFFFull);
         } else {
           uint64_t kp = K + std::max<uint64_t>(1024, K / 8);
           uint64_t delta = std::max<uint64_t>(2 * kp, 32768);
           // room for the first wave of tiles that run before any threshold exists (all resident CTAs x one tile)
-          uint64_t cap = std::min<uint64_t>((uint64_t)tmp.n_lr, 16 * kp + (4u << 20));
+          uint64_t cap = std::min<uint64_t>((uint64_t)s.n_lr, 16 * kp + (4u << 20));
           if (cap > 0xFFFFFFF0ull) return set_error(LDW_ERR_UNSUPPORTED, "long-range candidate buffer exceeds 2^32 entries");
           s.kprime = (uint32_t)kp; s.delta = (uint32_t)delta; s.cap = (uint32_t)cap;
         }
@@ -1048,77 +1082,48 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
         sum_keep += K;
       }
     }
+    kept_cap = 2 * sum_keep + (1u << 20);
+    return 0;
   }
-  const uint64_t kept_cap = 2 * sum_keep + (1u << 20);
 
-  // ---- device workspace
-  for (auto& l : W->lr) {
-    LDW_TRY(l.cand.ensure(max_cap * sizeof(Cand)));
-    LDW_TRY(l.mi64.ensure(max_cap * 8));
-    LDW_TRY(l.vcand.ensure(max_cap * sizeof(Cand)));
-    LDW_TRY(l.state.ensure(64));
-    LDW_TRY(l.hist.ensure(MI_HIST_BINS * 4));
-    l.used = false; l.chain_valid = false;
+  int reserve_workspace() {
+    for (auto& l : W->lr) {
+      LDW_TRY(l.cand.ensure(max_cap * sizeof(Cand)));
+      LDW_TRY(l.mi64.ensure(max_cap * 8));
+      LDW_TRY(l.vcand.ensure(max_cap * sizeof(Cand)));
+      LDW_TRY(l.state.ensure(64));
+      LDW_TRY(l.hist.ensure(MI_HIST_BINS * 4));
+      l.used = false; l.chain_valid = false;
+    }
+    LDW_TRY(W->d_state.ensure(64));
+    LDW_TRY(W->h_results.ensure(std::max<size_t>(blocks.size(), 1) * sizeof(BlockResult)));
+    LDW_TRY(W->h_pub.ensure(64));
+    memset(W->h_results.p, 0, std::max<size_t>(blocks.size(), 1) * sizeof(BlockResult));
+    LDW_TRY(W->d_sr_f32.ensure((size_t)std::max<int64_t>(total_sr, 1) * 4));
+    LDW_TRY(W->d_kept_key.ensure(kept_cap * 8));
+    LDW_TRY(W->d_kept_gi.ensure(kept_cap * 4));
+    LDW_TRY(W->d_kept_gj.ensure(kept_cap * 4));
+    LDW_TRY(W->d_kept_mi.ensure(kept_cap * 8));
+    LDW_TRY(W->d_kept_count.ensure(16));
+    if (sr_rows) LDW_TRY(W->d_sr.ensure(total_sr));
+    LDW_CUDA(cudaMemsetAsync(W->d_kept_count.p, 0, 16, st));
+    // Threshold seed for the next blocks: ONE word, overwritten by every selection and read by every block's begin
+    // kernel, whichever selection finished last (usually one or two blocks back).  The value read only steers how many
+    // candidates get collected -- results do not depend on it (the selection verifies completeness and is exact) -- so
+    // the unordered read across the two streams is harmless; zero (nothing selected yet) means "collect from zero".
+    d_chain = W->d_state.as<uint32_t>() + 8;
+    LDW_CUDA(cudaMemsetAsync(W->d_state.p, 0, 64, st));
+    P->ctx->dev_sr.n = -1;
+    if (sr_to_host) {
+      if (!shared && sr_rows) LDW_TRY(hsr.ensure(total_sr));
+      LDW_TRY(ev_blk.create(cudaEventDisableTiming));
+    }
+    return 0;
   }
-  LDW_TRY(W->d_state.ensure(64));
-  LDW_TRY(W->h_results.ensure(std::max<size_t>(blocks.size(), 1) * sizeof(BlockResult)));
-  LDW_TRY(W->h_pub.ensure(64));
-  memset(W->h_results.p, 0, std::max<size_t>(blocks.size(), 1) * sizeof(BlockResult));
-  LDW_TRY(W->d_sr_f32.ensure((size_t)std::max<int64_t>(total_sr, 1) * 4));
-  LDW_TRY(W->d_kept_key.ensure(kept_cap * 8));
-  LDW_TRY(W->d_kept_gi.ensure(kept_cap * 4));
-  LDW_TRY(W->d_kept_gj.ensure(kept_cap * 4));
-  LDW_TRY(W->d_kept_mi.ensure(kept_cap * 8));
-  LDW_TRY(W->d_kept_count.ensure(16));
-  const bool sr_rows = !(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_LR_ONLY));  // short-range link columns wanted at all
-  if (sr_rows) LDW_TRY(W->d_sr.ensure(total_sr));
-  LDW_CUDA(cudaMemsetAsync(W->d_kept_count.p, 0, 16, st));
-  uint32_t* d_kept_overflow = W->d_state.as<uint32_t>() + 3;
-  // Threshold seed for the next blocks: ONE word, overwritten by every selection and read by every block's begin
-  // kernel, whichever selection finished last (usually one or two blocks back).  The value read only steers how many
-  // candidates get collected -- results do not depend on it (the selection verifies completeness and is exact) -- so
-  // the unordered read across the two streams is harmless; zero (nothing selected yet) means "collect from zero".
-  uint32_t* d_chain2 = W->d_state.as<uint32_t>() + 8;
-  LDW_CUDA(cudaMemsetAsync(W->d_state.p, 0, 64, st));
-  cudaStream_t sst = P->ctx->select_stream;
 
-  const bool want_host = !(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H));
-  const bool sr_to_host = want_host && !(flags & LDW_SCAN_SR_ON_DEVICE);  // short-range rows cross PCIe at all?
-  P->ctx->dev_sr.n = -1;
-  cudaStream_t cst = P->ctx->copy_stream;
-  cudaEvent_t ev_blk = nullptr;  // "this block's SR columns are materialised"
-  // short-range rows go to this context's pinned table, or -- multi-GPU -- straight to the group's table, every rank
-  // at the final offsets of its blocks (the table is complete when the last rank finishes: no merge pass)
-  HostLinks& hsr = shared ? *shared->h_sr : P->ctx->h_sr;
-  if (sr_to_host) {
-    if (!shared && sr_rows) LDW_TRY(hsr.ensure(total_sr));
-    LDW_CUDA(cudaEventCreateWithFlags(&ev_blk, cudaEventDisableTiming));
-  }
-  auto tpre = std::chrono::steady_clock::now();
-  LDW_CUDA(cudaEventRecord(ev0, st));
-  int64_t n_reruns = 0, n_launches = 0, n_scan_launches = 0, n_tiles = 0;
-  double exec_ops = 0, exec_mufu = 0;
-  std::vector<cudaEvent_t> kev;  // pairs of events around every scan-kernel launch
-  auto kev_cleanup = [&]() { for (auto e : kev) cudaEventDestroy(e); kev.clear(); };
-  int64_t dbg_block = -1;
-  {
-    const char* e = getenv("LDW_DBG_BLOCK");
-    if (e) dbg_block = atoll(e);
-  }
-  double host_prep_ms = 0;
-  int scan_reserve = 2;  // SMs left to the selection stream (presel, refine, select of earlier blocks); 1-3 within 1 % at C2
-  if (const char* e = getenv("LDW_SCAN_RESERVE")) scan_reserve = atoi(e);
-  // test hook: force every block's first attempt to start from this candidate threshold (a value above the true
-  // threshold makes the selection fail its completeness check and exercises the re-run path)
-  float force_seed = -1.f;
-  if (const char* e = getenv("LDW_DBG_FORCE_SEED")) force_seed = (float)atof(e);
-  // b: index into this rank's block list (output offsets, results); seq: position in the execution order (ring slots)
-  // margin of the long-range selection (pre-selection window and completeness test): sound while twice the fp32
-  // epilogue's error stays below it; the selection kernel measures that error per block and asks for a re-run with a
-  // wider margin when it does not (BlockResult.bad & 8)
-  double sel_margin0 = 4e-6;
-  if (const char* e = getenv("LDW_DBG_SEL_MARGIN")) sel_margin0 = atof(e);  // test hook: a tiny margin exercises that re-run
-  auto run_block = [&](size_t b, size_t seq, int force_emit_all, uint32_t cap_override, bool use_chain, double sel_margin) -> int {
+  // Enqueues one block: host tables, upload, scan launch(es), long-range selection on the select stream, short-range
+  // columns and their copy to the host.  b: index into `blocks`; seq: position in the execution order (ring slots).
+  int run_block(size_t b, size_t seq, const Attempt& a) {
     Sel& s = sel[b];
     if (s.skip) return 0;
     int slot = (int)(seq % ScanWS::RING);
@@ -1128,13 +1133,12 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
     if (D.used) LDW_CUDA(cudaEventSynchronize(D.done));
     if (D.used2) { LDW_CUDA(cudaEventSynchronize(D.done2)); D.used2 = false; }
     ScanWS::LrBuf& L = W->lr[seq % ScanWS::NLR];
-    uint32_t* d_count = L.state.as<uint32_t>();
+    uint32_t* d_count = L.state.as<uint32_t>();  // state: count, tcand, overflow, -, -, vcount
     uint32_t* d_tcand = d_count + 1;
     uint32_t* d_overflow = d_count + 2;
-    uint32_t* d_chain = d_chain2;
-    auto hp0 = std::chrono::steady_clock::now();
+    auto hp0 = clock::now();
     int e;
-    if (seq == 0 && first_guess == (int64_t)b && first_rc >= 0 && first_rc <= 1 && !force_emit_all && !cap_override) {
+    if (seq == 0 && first_guess == (int64_t)b && first_rc >= 0 && first_rc <= 1 && !a.force_emit_all && !a.cap_override) {
       e = first_rc;  // built during pass 1
       first_rc = -1;
     } else {
@@ -1145,7 +1149,7 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
     LDW_TRY(upload_block(P->ctx->upload_stream, D, H));
     LDW_CUDA(cudaEventRecord(D.uploaded, P->ctx->upload_stream));
     LDW_CUDA(cudaStreamWaitEvent(st, D.uploaded, 0));
-    host_prep_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - hp0).count();
+    host_prep_ms += std::chrono::duration<double, std::milli>(clock::now() - hp0).count();
     D.used = true;
     ScanParams sp;
     fill_scan_params(P, D, H, cfg, sp);
@@ -1156,56 +1160,46 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
       sp.dbg = W->d_dbg.as<unsigned long long>();
     }
     const bool lr = !sr_only && s.n_lr > 0;
-    const int emit_all = force_emit_all || s.emit_all;
-    uint32_t cap = cap_override ? cap_override : s.cap;
+    const int emit_all = a.force_emit_all || s.emit_all;
+    const uint32_t cap = a.cap_override ? a.cap_override : s.cap;
     if (lr) {
       // this buffer's previous selection (three blocks earlier) must be done before its counters are cleared
       if (L.used) LDW_CUDA(cudaStreamWaitEvent(st, L.sel_done, 0));
       const int n_pilot = (int)H.tiles.size() - H.n_real_tiles;
-      if (seq == 0 && use_chain && !emit_all && n_pilot > 0) {
+      if (seq == 0 && a.use_chain && !emit_all && n_pilot > 0) {
         // first block of the call: nothing has been selected yet, so estimate its threshold from a pilot sample
         mi_block_begin_kernel<<<1, 256, 0, st>>>(d_count, L.hist.as<uint32_t>(), d_chain, 0);
         ScanParams pp = sp;
         pp.tiles = D.tiles.as<TileDesc>() + H.n_real_tiles;
         pp.n_tiles = n_pilot;
-        pp.cand = L.cand.as<Cand>(); pp.cand_cap = cap; pp.cand_count = d_count; pp.tcand_bits = d_tcand;
-        pp.hist = L.hist.as<uint32_t>(); pp.kprime = s.kprime; pp.delta = s.delta ? s.delta : 1; pp.overflow = d_overflow;
-        pp.emit_all = 1;
+        arm_collection(pp, L, s, cap, 1);
         pp.dbg = nullptr;
         LDW_TRY(launch_scan(P, pp, st, 0));
         mi_pilot_seed_kernel<<<1, 1024, 0, st>>>(L.cand.as<Cand>(), d_count, cap, (unsigned long long)s.k_lo, (double)s.n_lr, d_chain);
         LDW_CUDA(cudaGetLastError());
         n_launches += 3;
       }
-      if (force_seed >= 0.f && use_chain && !emit_all) {
+      if (force_seed >= 0.f && a.use_chain && !emit_all) {
         static_assert(sizeof(float) == 4, "float bits");
         LDW_CUDA(cudaMemcpyAsync(d_chain, &force_seed, 4, cudaMemcpyHostToDevice, st));
         LDW_CUDA(cudaStreamSynchronize(st));
       }
-      mi_block_begin_kernel<<<1, 256, 0, st>>>(d_count, L.hist.as<uint32_t>(), d_chain, (use_chain && !emit_all) ? 1 : 0);
+      mi_block_begin_kernel<<<1, 256, 0, st>>>(d_count, L.hist.as<uint32_t>(), d_chain, (a.use_chain && !emit_all) ? 1 : 0);
       LDW_CUDA(cudaGetLastError());
       n_launches++;
-      sp.cand = L.cand.as<Cand>();
-      sp.cand_cap = cap;
-      sp.cand_count = d_count;
-      sp.tcand_bits = d_tcand;
-      sp.hist = L.hist.as<uint32_t>();
-      sp.kprime = s.kprime;
-      sp.delta = s.delta ? s.delta : 1;
-      sp.overflow = d_overflow;
-      sp.emit_all = emit_all;
+      arm_collection(sp, L, s, cap, emit_all);
     } else {
       sp.sr_only = 1;  // nothing long-range to collect in this block
     }
     if (sp.n_tiles > 0) {
-      cudaEvent_t k0, k1;
-      LDW_CUDA(cudaEventCreate(&k0));
-      LDW_CUDA(cudaEventCreate(&k1));
-      kev.push_back(k0);
-      kev.push_back(k1);
+      Event k0, k1;
+      LDW_TRY(k0.create());
+      LDW_TRY(k1.create());
       LDW_CUDA(cudaEventRecord(k0, st));
       LDW_TRY(launch_scan(P, sp, st, lr ? scan_reserve : 0));
       LDW_CUDA(cudaEventRecord(k1, st));
+      kev.push_back(std::move(k0));
+      kev.push_back(std::move(k1));
       n_launches++; n_scan_launches++;
       n_tiles += sp.n_tiles;
       for (int32_t ti = 0; ti < H.n_real_tiles; ti++) {  // 4 K-passes x 2 ops/MAC x 128 rows x (PA*PB*NJ) columns x Kpad
@@ -1226,7 +1220,7 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
       RefineParams R = make_refine_params(P, D, H, cfg);
       // candidates that can reach the exact K-th largest value (fp32 pre-selection), then their fp64 refinement
       n_launches++;
-      mi_presel_kernel<<<1, 1024, 0, sst>>>(L.cand.as<Cand>(), d_count, cap, d_tcand, emit_all, (unsigned long long)s.k_lo, (float)sel_margin,
+      mi_presel_kernel<<<1, 1024, 0, sst>>>(L.cand.as<Cand>(), d_count, cap, d_tcand, emit_all, (unsigned long long)s.k_lo, (float)a.sel_margin,
                                            L.vcand.as<Cand>(), d_count + 5);
       LDW_CUDA(cudaGetLastError());
       mi_refine_list_kernel<<<P->ctx->num_sms * 4, 32 * REFINE_WARPS, 0, sst>>>(R, L.vcand.as<Cand>(), d_count + 5, L.mi64.as<double>());
@@ -1236,12 +1230,12 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
       q.cand = L.vcand.as<Cand>(); q.mi64 = L.mi64.as<double>(); q.vcount = d_count + 5; q.count = d_count; q.cap = cap;
       q.overflow = d_overflow; q.tcand_bits = d_tcand; q.emit_all = emit_all;
       q.k_lo = s.k_lo; q.k_hi = s.k_hi; q.h = s.h; q.interpolate = s.interp;
-      q.tol_safe = sel_margin; q.tol_border = 1e-9;
+      q.tol_safe = a.sel_margin; q.tol_border = 1e-9;
       q.from_idx = D.from_idx.as<int32_t>(); q.to_idx = D.to_idx.as<int32_t>();
       q.nf = H.nf; q.nt = H.nt; q.diag = H.diag; q.block = (int32_t)blocks[b].index;
       q.kept_key = W->d_kept_key.as<uint64_t>(); q.kept_gi = W->d_kept_gi.as<int32_t>(); q.kept_gj = W->d_kept_gj.as<int32_t>();
       q.kept_mi = W->d_kept_mi.as<double>(); q.kept_count = W->d_kept_count.as<unsigned long long>(); q.kept_cap = kept_cap;
-      q.kept_overflow = d_kept_overflow;
+      q.kept_overflow = W->d_state.as<uint32_t>() + 3;
       q.chain_bits = d_chain;
       q.result = W->h_results.as<BlockResult>() + b;
       mi_select_kernel<<<1, 1024, 0, sst>>>(q);
@@ -1257,14 +1251,14 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
       m.col = D.colinfo.as<ColInfo>(); m.from_idx = D.from_idx.as<int32_t>(); m.to_idx = D.to_idx.as<int32_t>();
       m.pos = P->d_pos.as<int32_t>(); m.paint = P->d_paint.as<int32_t>();
       m.sr_mi = W->d_sr_f32.as<float>() + s.sr_base;
-      m.nf = H.nf; m.nt = H.nt; m.diag = H.diag; m.block = (int32_t)blocks[b].index; m.g = (int64_t)g;
+      m.nf = H.nf; m.nt = H.nt; m.diag = H.diag; m.block = (int32_t)blocks[b].index; m.g = (int64_t)cfg.g;
       m.o_pos1 = W->d_sr.pos1.as<int32_t>() + s.sr_base; m.o_pos2 = W->d_sr.pos2.as<int32_t>() + s.sr_base;
       m.o_c1 = W->d_sr.c1.as<int32_t>() + s.sr_base; m.o_c2 = W->d_sr.c2.as<int32_t>() + s.sr_base;
       m.o_len = W->d_sr.len.as<int32_t>() + s.sr_base; m.o_blk = W->d_sr.blk.as<int32_t>() + s.sr_base;
       m.o_mi = W->d_sr.mi.as<double>() + s.sr_base;
       mi_sr_materialize_kernel<<<H.nt, 128, 0, st>>>(m);
       LDW_CUDA(cudaGetLastError());
-      if (flags & LDW_SCAN_SR_EXACT) {  // fp64 MI over the fp32-derived column, before the rows leave for the host
+      if (cfg.flags & LDW_SCAN_SR_EXACT) {  // fp64 MI over the fp32-derived column, before the rows leave for the host
         n_launches++;
         mi_sr_exact_kernel<<<H.nt, 32 * REFINE_WARPS, 0, st>>>(m, make_refine_params(P, D, H, cfg));
         LDW_CUDA(cudaGetLastError());
@@ -1273,196 +1267,183 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
         // copy this block's finished rows to the host while the next blocks are being scanned
         LDW_CUDA(cudaEventRecord(ev_blk, st));
         LDW_CUDA(cudaStreamWaitEvent(cst, ev_blk, 0));
-        HostLinks& h = hsr;
-        const size_t o = (size_t)s.sr_hbase, nb4 = (size_t)s.n_sr * 4, nb8 = (size_t)s.n_sr * 8;
-        LDW_CUDA(cudaMemcpyAsync(h.pos1.as<int32_t>() + o, m.o_pos1, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.pos2.as<int32_t>() + o, m.o_pos2, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.c1.as<int32_t>() + o, m.o_c1, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.c2.as<int32_t>() + o, m.o_c2, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.len.as<int32_t>() + o, m.o_len, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.blk.as<int32_t>() + o, m.o_blk, nb4, cudaMemcpyDeviceToHost, cst));
-        LDW_CUDA(cudaMemcpyAsync(h.mi.as<double>() + o, m.o_mi, nb8, cudaMemcpyDeviceToHost, cst));
+        for (int c = 0; c < DevLinks::NCOL; c++) {
+          const size_t el = DevLinks::elem(c);
+          LDW_CUDA(cudaMemcpyAsync(hsr.col(c).as<char>() + s.sr_hbase * el, W->d_sr.col(c).as<char>() + s.sr_base * el,
+                                   (size_t)s.n_sr * el, cudaMemcpyDeviceToHost, cst));
+        }
       }
     }
     LDW_CUDA(cudaEventRecord(D.done, st));
     return 0;
-  };
-  // Execution order: blocks that hold short-range links first, so their (large) link columns cross PCIe while the
-  // long-range-only blocks are still being scanned.  Output order is unaffected: short-range rows have fixed
-  // offsets and the kept long-range rows are sorted by (block, row rank) afterwards.
-  std::vector<size_t> order;
-  for (size_t b = 0; b < blocks.size(); b++) if (sel[b].n_sr > 0) order.push_back(b);
-  for (size_t b = 0; b < blocks.size(); b++) if (!(sel[b].n_sr > 0)) order.push_back(b);
-  for (size_t k = 0; k < order.size(); k++) LDW_TRY(run_block(order[k], k, 0, 0, true, sel_margin0));
-  for (auto& l : W->lr)
-    if (l.used) LDW_CUDA(cudaStreamWaitEvent(st, l.sel_done, 0));  // join the select stream
-  LDW_CUDA(cudaEventRecord(ev1, st));
-  const bool dbg_timing = getenv("LDW_DBG_TIMING") != nullptr;
-  auto tp0 = std::chrono::steady_clock::now();
-  auto lap = [&](const char* what) {
-    if (!dbg_timing) return;
-    cudaStreamSynchronize(st);
-    auto t = std::chrono::steady_clock::now();
-    fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(t - tp0).count());
-    tp0 = t;
-  };
-  if (dbg_timing) fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", "sizes + workspace (host)", std::chrono::duration<double, std::milli>(tpre - t_entry).count());
-  if (dbg_timing) fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", "submit blocks (host)", std::chrono::duration<double, std::milli>(tp0 - tpre).count());
-  lap("drain blocks");
+  }
 
-  // ---- verify the long-range selection of every block; re-run the (rare) blocks whose candidate set is not
-  //      provably complete with a plain "collect everything" pass
-  LDW_CUDA(cudaStreamSynchronize(st));
-  P->results.assign(W->h_results.as<BlockResult>(), W->h_results.as<BlockResult>() + blocks.size());
-  if (!sr_only) {
-    for (size_t b = 0; b < blocks.size(); b++) {
-      if (sel[b].skip || sel[b].n_lr == 0) continue;
-      if (P->results[b].bad) {
-        // second attempt: no chained seed (collect from zero, the histogram places the threshold); last resort:
-        // collect every long-range pair of the block
-        double margin = sel_margin0;
-        for (int attempt = 0; attempt < 2 && P->results[b].bad; attempt++) {
-          n_reruns++;
-          // measured epilogue error too large for the margin: widen it to 8x the observation (the test wants 4x)
-          if (P->results[b].bad & 8) margin = std::max(std::max(margin, 4e-6), 8.0 * (double)P->results[b].eps_obs);
-          uint32_t cap = 0;
-          if (attempt == 1) {
-            if ((uint64_t)sel[b].n_lr > 0xFFFFFFF0ull) return set_error(LDW_ERR_UNSUPPORTED, "block %lld needs an exhaustive long-range pass over more than 2^32 links", (long long)blocks[b].index);
-            cap = (uint32_t)sel[b].n_lr;
-            ScanWS::LrBuf& L = W->lr[0];
-            LDW_TRY(L.cand.ensure((size_t)cap * sizeof(Cand)));
-            LDW_TRY(L.mi64.ensure((size_t)cap * 8));
-            LDW_TRY(L.vcand.ensure((size_t)cap * sizeof(Cand)));
+  // Every block once, then the select stream joined.  Execution order: blocks that hold short-range links first, so
+  // their (large) link columns cross PCIe while the long-range-only blocks are still being scanned.  Output order is
+  // unaffected: short-range rows have fixed offsets and the kept long-range rows are sorted by (block, row rank) afterwards.
+  int submit_blocks() {
+    tpre = clock::now();
+    LDW_CUDA(cudaEventRecord(ev0, st));
+    std::vector<size_t> order;
+    for (size_t b = 0; b < blocks.size(); b++) if (sel[b].n_sr > 0) order.push_back(b);
+    for (size_t b = 0; b < blocks.size(); b++) if (!(sel[b].n_sr > 0)) order.push_back(b);
+    for (size_t k = 0; k < order.size(); k++) LDW_TRY(run_block(order[k], k, Attempt{false, 0, true, sel_margin0}));
+    for (auto& l : W->lr)
+      if (l.used) LDW_CUDA(cudaStreamWaitEvent(st, l.sel_done, 0));  // join the select stream
+    LDW_CUDA(cudaEventRecord(ev1, st));
+    tp0 = clock::now();
+    if (dbg_timing) fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", "sizes + workspace (host)", std::chrono::duration<double, std::milli>(tpre - t_entry).count());
+    if (dbg_timing) fprintf(stderr, "ldw timing: %-28s %8.3f ms\n", "submit blocks (host)", std::chrono::duration<double, std::milli>(tp0 - tpre).count());
+    lap("drain blocks");
+    return 0;
+  }
+
+  // Verifies the long-range selection of every block; re-runs the (rare) blocks whose candidate set is not provably
+  // complete with a plain "collect everything" pass.
+  int verify_and_rerun() {
+    LDW_CUDA(cudaStreamSynchronize(st));
+    P->results.assign(W->h_results.as<BlockResult>(), W->h_results.as<BlockResult>() + blocks.size());
+    if (!sr_only) {
+      for (size_t b = 0; b < blocks.size(); b++) {
+        if (sel[b].skip || sel[b].n_lr == 0) continue;
+        if (P->results[b].bad) {
+          // second attempt: no chained seed (collect from zero, the histogram places the threshold); last resort:
+          // collect every long-range pair of the block
+          double margin = sel_margin0;
+          for (int attempt = 0; attempt < 2 && P->results[b].bad; attempt++) {
+            n_reruns++;
+            // measured epilogue error too large for the margin: widen it to 8x the observation (the test wants 4x)
+            if (P->results[b].bad & 8) margin = std::max(std::max(margin, 4e-6), 8.0 * (double)P->results[b].eps_obs);
+            uint32_t cap = 0;
+            if (attempt == 1) {
+              if ((uint64_t)sel[b].n_lr > 0xFFFFFFF0ull) return set_error(LDW_ERR_UNSUPPORTED, "block %lld needs an exhaustive long-range pass over more than 2^32 links", (long long)blocks[b].index);
+              cap = (uint32_t)sel[b].n_lr;
+              ScanWS::LrBuf& L = W->lr[0];
+              LDW_TRY(L.cand.ensure((size_t)cap * sizeof(Cand)));
+              LDW_TRY(L.mi64.ensure((size_t)cap * 8));
+              LDW_TRY(L.vcand.ensure((size_t)cap * sizeof(Cand)));
+            }
+            LDW_TRY(run_block(b, 0, Attempt{attempt == 1, cap, false, margin}));
+            LDW_CUDA(cudaStreamWaitEvent(st, W->lr[0].sel_done, 0));
+            LDW_CUDA(cudaStreamSynchronize(st));
+            P->results[b] = W->h_results.as<BlockResult>()[b];
           }
-          LDW_TRY(run_block(b, 0, attempt == 1, cap, false, margin));
-          LDW_CUDA(cudaStreamWaitEvent(st, W->lr[0].sel_done, 0));
-          LDW_CUDA(cudaStreamSynchronize(st));
-          P->results[b] = W->h_results.as<BlockResult>()[b];
+          if (P->results[b].bad) return set_error(LDW_ERR_INTERNAL, "long-range selection failed for block %lld (flags %u)", (long long)blocks[b].index, P->results[b].bad);
         }
-        if (P->results[b].bad) return set_error(LDW_ERR_INTERNAL, "long-range selection failed for block %lld (flags %u)", (long long)blocks[b].index, P->results[b].bad);
       }
     }
+    lap("results + reruns");
+    return 0;
   }
-  lap("results + reruns");
-  unsigned long long n_kept = 0;
-  uint32_t state[4] = {0, 0, 0, 0};
-  publish_kernel<<<1, 1, 0, st>>>(W->d_kept_count.as<unsigned long long>(), W->d_state.as<uint32_t>(), W->h_pub.as<unsigned long long>());
-  LDW_CUDA(cudaGetLastError());
-  LDW_CUDA(cudaStreamSynchronize(st));
-  n_kept = W->h_pub.as<unsigned long long>()[0];
-  state[3] = (uint32_t)W->h_pub.as<unsigned long long>()[1];
-  if (state[3] || n_kept > kept_cap) return set_error(LDW_ERR_UNSUPPORTED, "more long-range links pass their block thresholds (%llu) than the output buffer holds (%llu): massive ties at the threshold", n_kept, (unsigned long long)kept_cap);
 
-  // ---- long-range rows into reference order (block, then row order inside the block)
-  int64_t n_border = 0;
-  for (auto& r : P->results) n_border += r.n_border;
-  if (n_kept > 0 && !(flags & LDW_SCAN_NO_LINKS)) {
-    n_launches += 2 + 4;  // iota, materialise, radix-sort passes (library)
-    LDW_TRY(W->d_keys_sorted.ensure(n_kept * 8));
-    LDW_TRY(W->d_order_in.ensure(n_kept * 4));
-    LDW_TRY(W->d_order_out.ensure(n_kept * 4));
-    iota_u32_kernel<<<(unsigned)((n_kept + 255) / 256), 256, 0, st>>>(W->d_order_in.as<uint32_t>(), (int64_t)n_kept);
-    size_t tmp_bytes = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, W->d_kept_key.as<uint64_t>(), W->d_keys_sorted.as<uint64_t>(),
-                                    W->d_order_in.as<uint32_t>(), W->d_order_out.as<uint32_t>(), (int)n_kept, 0, 64, st);
-    LDW_TRY(W->d_sort_tmp.ensure(tmp_bytes));
-    LDW_CUDA(cub::DeviceRadixSort::SortPairs(W->d_sort_tmp.p, tmp_bytes, W->d_kept_key.as<uint64_t>(), W->d_keys_sorted.as<uint64_t>(),
-                                             W->d_order_in.as<uint32_t>(), W->d_order_out.as<uint32_t>(), (int)n_kept, 0, 64, st));
-    LDW_TRY(W->d_lr.ensure((int64_t)n_kept));
-    mi_lr_materialize_kernel<<<(unsigned)((n_kept + 255) / 256), 256, 0, st>>>(
-        W->d_order_out.as<uint32_t>(), W->d_keys_sorted.as<uint64_t>(), W->d_kept_gi.as<int32_t>(), W->d_kept_gj.as<int32_t>(),
-        W->d_kept_mi.as<double>(), P->d_pos.as<int32_t>(), P->d_paint.as<int32_t>(), (int64_t)n_kept, (int64_t)g,
-        W->d_lr.pos1.as<int32_t>(), W->d_lr.pos2.as<int32_t>(), W->d_lr.c1.as<int32_t>(), W->d_lr.c2.as<int32_t>(),
-        W->d_lr.len.as<int32_t>(), W->d_lr.mi.as<double>(), W->d_lr.blk.as<int32_t>());
+  // The kept long-range rows into reference order (block, then row order inside the block), as link columns.
+  int sort_long_range() {
+    publish_kernel<<<1, 1, 0, st>>>(W->d_kept_count.as<unsigned long long>(), W->d_state.as<uint32_t>(), W->h_pub.as<unsigned long long>());
     LDW_CUDA(cudaGetLastError());
-  }
-  LDW_CUDA(cudaEventRecord(ev2, st));
-  lap("lr sort + materialise");
-
-  // ---- device -> pinned host
-  P->ctx->h_sr.n = 0; P->ctx->h_lr.n = 0; P->ctx->h_border.n = 0;
-  if (!(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H))) {
-    auto d2h = [&](HostLinks& h, DevLinks& d, int64_t m) -> int {
-      LDW_TRY(h.ensure(m));
-      h.n = m;
-      if (m == 0) return 0;
-      LDW_CUDA(cudaMemcpyAsync(h.pos1.p, d.pos1.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.pos2.p, d.pos2.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.c1.p, d.c1.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.c2.p, d.c2.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.len.p, d.len.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.blk.p, d.blk.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(h.mi.p, d.mi.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
-      return 0;
-    };
-    if (!shared) P->ctx->h_sr.n = (sr_rows && sr_to_host) ? total_sr : 0;  // short-range rows were streamed out block by block on the copy stream
-    LDW_TRY(d2h(P->ctx->h_lr, W->d_lr, (int64_t)n_kept));
-  }
-  LDW_CUDA(cudaEventRecord(ev3, st));
-  LDW_CUDA(cudaStreamSynchronize(st));
-  lap("lr d2h");
-  if (sr_to_host) LDW_CUDA(cudaStreamSynchronize(cst));
-  lap("copy stream drain");
-  if (ev_blk) cudaEventDestroy(ev_blk);
-
-  // borderline list: kept-or-not candidates within tol of their block threshold are reported by count per block;
-  // the explicit rows are the LR rows whose MI is within tol of the block threshold
-  if (borderline_out) {
-    std::vector<int64_t> idx;
-    const int32_t* blkcol = P->ctx->h_lr.blk.as<int32_t>();
-    const double* micol = P->ctx->h_lr.mi.as<double>();
-    std::vector<double> thr_by_index(nblk_total, NAN);
-    for (size_t b = 0; b < blocks.size(); b++)
-      if (!sel[b].skip && sel[b].n_lr > 0 && !sr_only) thr_by_index[blocks[b].index] = P->results[b].thr;
-    for (int64_t i = 0; i < P->ctx->h_lr.n; i++)
-      if (std::fabs(micol[i] - thr_by_index[blkcol[i]]) <= 1e-9) idx.push_back(i);
-    LDW_TRY(P->ctx->h_border.ensure((int64_t)idx.size()));
-    P->ctx->h_border.n = (int64_t)idx.size();
-    for (size_t k = 0; k < idx.size(); k++) {
-      int64_t i = idx[k];
-      P->ctx->h_border.pos1.as<int32_t>()[k] = P->ctx->h_lr.pos1.as<int32_t>()[i];
-      P->ctx->h_border.pos2.as<int32_t>()[k] = P->ctx->h_lr.pos2.as<int32_t>()[i];
-      P->ctx->h_border.c1.as<int32_t>()[k] = P->ctx->h_lr.c1.as<int32_t>()[i];
-      P->ctx->h_border.c2.as<int32_t>()[k] = P->ctx->h_lr.c2.as<int32_t>()[i];
-      P->ctx->h_border.len.as<int32_t>()[k] = P->ctx->h_lr.len.as<int32_t>()[i];
-      P->ctx->h_border.blk.as<int32_t>()[k] = blkcol[i];
-      P->ctx->h_border.mi.as<double>()[k] = micol[i];
+    LDW_CUDA(cudaStreamSynchronize(st));
+    n_kept = W->h_pub.as<unsigned long long>()[0];
+    const uint32_t kept_overflow = (uint32_t)W->h_pub.as<unsigned long long>()[1];
+    if (kept_overflow || n_kept > kept_cap) return set_error(LDW_ERR_UNSUPPORTED, "more long-range links pass their block thresholds (%llu) than the output buffer holds (%llu): massive ties at the threshold", n_kept, (unsigned long long)kept_cap);
+    if (n_kept > 0 && !(cfg.flags & LDW_SCAN_NO_LINKS)) {
+      n_launches += 2 + 4;  // iota, materialise, radix-sort passes (library)
+      LDW_TRY(W->d_keys_sorted.ensure(n_kept * 8));
+      LDW_TRY(W->d_order_in.ensure(n_kept * 4));
+      LDW_TRY(W->d_order_out.ensure(n_kept * 4));
+      iota_u32_kernel<<<(unsigned)((n_kept + 255) / 256), 256, 0, st>>>(W->d_order_in.as<uint32_t>(), (int64_t)n_kept);
+      size_t tmp_bytes = 0;
+      cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, W->d_kept_key.as<uint64_t>(), W->d_keys_sorted.as<uint64_t>(),
+                                      W->d_order_in.as<uint32_t>(), W->d_order_out.as<uint32_t>(), (int)n_kept, 0, 64, st);
+      LDW_TRY(W->d_sort_tmp.ensure(tmp_bytes));
+      LDW_CUDA(cub::DeviceRadixSort::SortPairs(W->d_sort_tmp.p, tmp_bytes, W->d_kept_key.as<uint64_t>(), W->d_keys_sorted.as<uint64_t>(),
+                                               W->d_order_in.as<uint32_t>(), W->d_order_out.as<uint32_t>(), (int)n_kept, 0, 64, st));
+      LDW_TRY(W->d_lr.ensure((int64_t)n_kept));
+      mi_lr_materialize_kernel<<<(unsigned)((n_kept + 255) / 256), 256, 0, st>>>(
+          W->d_order_out.as<uint32_t>(), W->d_keys_sorted.as<uint64_t>(), W->d_kept_gi.as<int32_t>(), W->d_kept_gj.as<int32_t>(),
+          W->d_kept_mi.as<double>(), P->d_pos.as<int32_t>(), P->d_paint.as<int32_t>(), (int64_t)n_kept, (int64_t)cfg.g,
+          W->d_lr.pos1.as<int32_t>(), W->d_lr.pos2.as<int32_t>(), W->d_lr.c1.as<int32_t>(), W->d_lr.c2.as<int32_t>(),
+          W->d_lr.len.as<int32_t>(), W->d_lr.mi.as<double>(), W->d_lr.blk.as<int32_t>());
+      LDW_CUDA(cudaGetLastError());
     }
-    P->ctx->h_border.fill(borderline_out);
+    LDW_CUDA(cudaEventRecord(ev2, st));
+    lap("lr sort + materialise");
+    return 0;
   }
-  if (flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H)) {
-    if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = total_sr; }
-    if (lr_out) { memset(lr_out, 0, sizeof(*lr_out)); lr_out->n = (int64_t)n_kept; }
-  } else {
-    if (shared || !sr_to_host) { if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = sr_rows ? total_sr : 0; } }
-    else P->ctx->h_sr.fill(sr_out);
 
-    P->ctx->h_lr.fill(lr_out);
+  // Device -> pinned host, the borderline rows, and every output of the call but the stats.
+  int hand_back(ldw_links* sr_out, ldw_links* lr_out, ldw_links* borderline_out, double* thr_out, double* prob_out) {
+    ldw_ctx* ctx = P->ctx;
+    const bool no_host = (cfg.flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H)) != 0;
+    ctx->h_sr.n = 0; ctx->h_lr.n = 0; ctx->h_border.n = 0;
+    if (!no_host) {
+      if (!shared) ctx->h_sr.n = (sr_rows && sr_to_host) ? total_sr : 0;  // short-range rows were streamed out block by block on the copy stream
+      LDW_TRY(ctx->h_lr.ensure((int64_t)n_kept));
+      ctx->h_lr.n = (int64_t)n_kept;
+      if (n_kept > 0)
+        for (int c = 0; c < DevLinks::NCOL; c++)
+          LDW_CUDA(cudaMemcpyAsync(ctx->h_lr.col(c).p, W->d_lr.col(c).p, (size_t)n_kept * DevLinks::elem(c), cudaMemcpyDeviceToHost, st));
+    }
+    LDW_CUDA(cudaEventRecord(ev3, st));
+    LDW_CUDA(cudaStreamSynchronize(st));
+    lap("lr d2h");
+    if (sr_to_host) LDW_CUDA(cudaStreamSynchronize(cst));
+    lap("copy stream drain");
+
+    // borderline list: kept-or-not candidates within tol of their block threshold are reported by count per block;
+    // the explicit rows are the LR rows whose MI is within tol of the block threshold
+    if (borderline_out) {
+      std::vector<int64_t> idx;
+      const int32_t* blkcol = ctx->h_lr.blk.as<int32_t>();
+      const double* micol = ctx->h_lr.mi.as<double>();
+      std::vector<double> thr_by_index(nblk_total, NAN);
+      for (size_t b = 0; b < blocks.size(); b++)
+        if (!sel[b].skip && sel[b].n_lr > 0 && !sr_only) thr_by_index[blocks[b].index] = P->results[b].thr;
+      for (int64_t i = 0; i < ctx->h_lr.n; i++)
+        if (std::fabs(micol[i] - thr_by_index[blkcol[i]]) <= 1e-9) idx.push_back(i);
+      LDW_TRY(ctx->h_border.ensure((int64_t)idx.size()));
+      ctx->h_border.n = (int64_t)idx.size();
+      for (int c = 0; c < HostLinks::NCOL; c++) {
+        const size_t el = HostLinks::elem(c);
+        const char* src = ctx->h_lr.col(c).as<char>();
+        char* dst = ctx->h_border.col(c).as<char>();
+        for (size_t k = 0; k < idx.size(); k++) memcpy(dst + k * el, src + idx[k] * el, el);
+      }
+      ctx->h_border.fill(borderline_out);
+    }
+    if (no_host) {
+      if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = total_sr; }
+      if (lr_out) { memset(lr_out, 0, sizeof(*lr_out)); lr_out->n = (int64_t)n_kept; }
+    } else {
+      if (shared || !sr_to_host) { if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = sr_rows ? total_sr : 0; } }
+      else ctx->h_sr.fill(sr_out);
+
+      ctx->h_lr.fill(lr_out);
+    }
+    if (sr_rows && n_parts == 1) {  // the whole job's table is in this context's device memory, in reference order
+      ldw_ctx::DevSr& d = ctx->dev_sr;
+      d.pos1 = W->d_sr.pos1.as<int32_t>(); d.pos2 = W->d_sr.pos2.as<int32_t>(); d.c1 = W->d_sr.c1.as<int32_t>();
+      d.c2 = W->d_sr.c2.as<int32_t>(); d.len = W->d_sr.len.as<int32_t>(); d.blk = W->d_sr.blk.as<int32_t>();
+      d.mi = W->d_sr.mi.as<double>();
+      d.n = total_sr;
+    }
+    for (size_t b = 0; b < blocks.size(); b++) {
+      if (sel[b].skip || sel[b].n_lr == 0 || sr_only) continue;
+      if (thr_out) thr_out[blocks[b].index] = P->results[b].thr;
+      if (prob_out) prob_out[blocks[b].index] = sel[b].prob;
+    }
+    return 0;
   }
-  if (sr_rows && n_parts == 1) {  // the whole job's table is in this context's device memory, in reference order
-    ldw_ctx::DevSr& d = P->ctx->dev_sr;
-    d.pos1 = W->d_sr.pos1.as<int32_t>(); d.pos2 = W->d_sr.pos2.as<int32_t>(); d.c1 = W->d_sr.c1.as<int32_t>();
-    d.c2 = W->d_sr.c2.as<int32_t>(); d.len = W->d_sr.len.as<int32_t>(); d.blk = W->d_sr.blk.as<int32_t>();
-    d.mi = W->d_sr.mi.as<double>();
-    d.n = total_sr;
-  }
-  for (size_t b = 0; b < blocks.size(); b++) {
-    if (sel[b].skip || sel[b].n_lr == 0 || sr_only) continue;
-    if (thr_out) thr_out[blocks[b].index] = P->results[b].thr;
-    if (prob_out) prob_out[blocks[b].index] = sel[b].prob;
-  }
-  if (stats_out) {
+
+  void fill_stats(ldw_scan_stats* stats_out) {
+    if (!stats_out) return;
     memset(stats_out, 0, sizeof(*stats_out));
     stats_out->n_blocks = (int64_t)blocks.size();
     stats_out->n_pairs = total_pairs;
     stats_out->n_sr = total_sr;
     stats_out->n_lr_total = sr_only ? 0 : total_lr;
     stats_out->n_lr_kept = (int64_t)n_kept;
-    stats_out->n_borderline = n_border;
-    {
-      int64_t nc = 0;
-      for (auto& r : P->results) nc += r.n_cand;
-      stats_out->n_candidates = nc;
+    for (auto& r : P->results) {
+      stats_out->n_borderline += r.n_border;
+      stats_out->n_candidates += r.n_cand;
     }
     stats_out->n_reruns = n_reruns;
     float a = 0, b = 0, c = 0;
@@ -1488,9 +1469,9 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
         cudaEventElapsedTime(&ms, kev[k], kev[k + 1]);
         gaps += ms;
         gmax = std::max<double>(gmax, ms);
-        char b[32];
-        snprintf(b, sizeof(b), " %.0f", 1e3 * ms);
-        detail += b;
+        char buf[32];
+        snprintf(buf, sizeof(buf), " %.0f", 1e3 * ms);
+        detail += buf;
       }
       float first = 0, last = 0;
       cudaEventElapsedTime(&first, ev0, kev[0]);
@@ -1504,14 +1485,15 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
     stats_out->exec_int8_ops = exec_ops;
     stats_out->t_host_prep_ms = host_prep_ms;
     stats_out->exec_mufu_ops = exec_mufu;
-    {
-      double em = 0;
-      for (size_t b = 0; b < blocks.size(); b++)
-        if (!sel[b].skip && sel[b].n_lr > 0 && !sr_only) em = std::max(em, (double)P->results[b].eps_obs);
-      stats_out->eps_obs_max = em;
-    }
+    double em = 0;
+    for (size_t k = 0; k < blocks.size(); k++)
+      if (!sel[k].skip && sel[k].n_lr > 0 && !sr_only) em = std::max(em, (double)P->results[k].eps_obs);
+    stats_out->eps_obs_max = em;
   }
-  if (dbg_block >= 0 && W->d_dbg.p) {
+
+  // LDW_DBG_BLOCK: the per-role cycle counters the scan kernel wrote for that block, averaged over its CTAs.
+  void print_dbg_block() {
+    if (dbg_block < 0 || !W->d_dbg.p) return;
     std::vector<unsigned long long> h(4096 * 16);
     cudaMemcpy(h.data(), W->d_dbg.p, h.size() * 8, cudaMemcpyDeviceToHost);
     double s[16] = {0};
@@ -1526,8 +1508,26 @@ int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain
               s[13] / nb / 1e3, s[6] / nb / 1e3, s[7] / nb / 1e3, s[8] / nb / 1e3, s[9] / nb / 1e3, s[10] / nb / 1e3, s[11] / nb / 1e3);
     }
   }
-  kev_cleanup();
-  cudaEventDestroy(ev0); cudaEventDestroy(ev1); cudaEventDestroy(ev2); cudaEventDestroy(ev3);
-  lap("borderline + stats (host)");
+};
+
+}  // namespace
+
+int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links, double lr_links_approx, int flags,
+                      int n_parts, int part, const ScanShared* shared, ldw_links* sr_out, ldw_links* lr_out,
+                      ldw_links* borderline_out, double* thr_out, double* prob_out, ldw_scan_stats* stats_out) {
+  if (!P) return set_error(LDW_ERR_ARG, "null plan");
+  const auto t_entry = std::chrono::steady_clock::now();
+  LDW_TRY(ctx_bind(P->ctx));
+  ScanRun R(P, ScanCfg{g, sr_dist, flags}, lr_retain_links, lr_links_approx, n_parts, shared, t_entry);
+  LDW_TRY(R.take_share(part, thr_out, prob_out));
+  LDW_TRY(R.size_blocks());
+  LDW_TRY(R.reserve_workspace());
+  LDW_TRY(R.submit_blocks());
+  LDW_TRY(R.verify_and_rerun());
+  LDW_TRY(R.sort_long_range());
+  LDW_TRY(R.hand_back(sr_out, lr_out, borderline_out, thr_out, prob_out));
+  R.fill_stats(stats_out);
+  R.print_dbg_block();
+  R.lap("borderline + stats (host)");
   return 0;
 }

@@ -17,8 +17,8 @@ rule says so), the same with ``return_parts=True`` (never fused; the whole dista
 ``DeviceGroup`` (the path of the benchmark's C3 configuration).  Counts, weights and distances must agree bit for bit.
 
 ``test_cases_reach_their_regime`` restates the path choice of ``hdw_device`` and fails if a case stops reaching the
-regime it is here for; it needs no GPU.  The class-matrix validation of ``ldw_hdw`` and ``ldw_group_load_codes`` is
-tested at the end.
+regime it is here for; it needs no GPU.  The class-matrix validation of ``ldw_hdw``, ``ldw_group_load_codes`` and
+``ldw_mi_plan_create`` is tested at the end.
 
 On one B200 the module runs in about a minute, most of it in the host reference at S ~ 6000.
 """
@@ -526,3 +526,21 @@ def test_group_load_codes_refuses_a_class_above_4(where, group):
     assert e.value.code == 1
     dist = reference_dist(good)
     check_case("after a refused matrix", good, (threshold_for(pick_thresh(dist, 50), len(good)),), group, dist)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("where", BAD_BODY + BAD_TAIL)
+def test_mi_plan_create_refuses_a_class_above_4(where):
+    import ldweaver_b200 as ldw
+    from ldweaver_b200 import _lib
+    good = _valid_codes()
+    n, S = good.shape
+    bad = good.copy()
+    bad.reshape(-1)[where] = 5
+    hdw, paint = np.full(S, 0.5), np.ones(n, dtype=np.int32)
+    with pytest.raises(_lib.LdwError, match="class 5 outside 0..4") as e:
+        ldw.MIPlan(ldw.snp_dat_from_codes(bad, np.arange(1, n + 1), n), hdw, paint, 128, device=0)
+    assert e.value.code == 1   # LDW_ERR_ARG
+    # the same context still builds a plan and scans a block with it
+    plan = ldw.MIPlan(ldw.snp_dat_from_codes(good, np.arange(1, n + 1), n), hdw, paint, 128, device=0)
+    assert plan.block_dense(0).shape == (n, n)
