@@ -50,17 +50,24 @@ enum {
 enum {
   LDW_SCAN_SR_ONLY = 1,   /* perform_SR_analysis_only = TRUE (R/computePairwiseMI.R:179-189, quirk Q12) */
   LDW_SCAN_IDEAL_Q = 2,   /* opt-out of quirk Q1: use 0.25*r_i*r_j on off-diagonal blocks too (NOT reference behaviour) */
-  LDW_SCAN_NO_LINKS = 4,  /* compute MI / thresholds only: no link columns are materialised or copied */
+  LDW_SCAN_NO_LINKS = 4,  /* compute MI / thresholds only: no link columns are materialised or copied.  The counts are those
+                             of LDW_SCAN_NO_D2H (sr_out->n = short-range links, lr_out->n = kept long-range links, NULL
+                             columns) and borderline_out is empty */
   LDW_SCAN_NO_D2H = 8,    /* materialise the link columns in device memory but do not copy them to the host
-                             (device-resident throughput measurement); link outputs come back with n rows and NULL pointers */
+                             (device-resident throughput measurement); link outputs come back with n rows and NULL pointers,
+                             and borderline_out empty (n = 0) even where stats_out->n_borderline > 0 */
   LDW_SCAN_SR_EXACT = 16, /* recompute the MI of every short-range link in fp64 (the reference's arithmetic) on the device,
                              block by block, before the rows are copied out (mi_sr_exact_kernel; also valid with
                              LDW_SCAN_SR_ONLY).  Parity-checked on the fixture in both modes (1e-12) */
   LDW_SCAN_SR_ON_DEVICE = 64, /* the short-range rows are materialised in device memory and STAY there (sr_out comes back with n rows
                              and NULL columns); long-range and borderline rows are copied as usual.  For ldw_sr_postprocess_dev,
                              which derives sr_links_red / the ARACNE check set from the device-resident table, so that the
-                             2.9 GB (616 x 100k) of short-range columns never cross PCIe */
-  LDW_SCAN_LR_ONLY = 32   /* no short-range link table (sr_out->n = 0): only the long-range rows, thresholds and statistics.
+                             2.9 GB (616 x 100k) of short-range columns never cross PCIe.  In ldw_group_mi_scan with more
+                             than one local member sr_out->n is the job's short-range count, the columns are NULL, and no
+                             device holds the whole table, so ldw_sr_postprocess_dev has none */
+  LDW_SCAN_LR_ONLY = 32   /* no short-range link table (sr_out->n = 0 with every other flag, LDW_SCAN_NO_D2H and
+                             LDW_SCAN_NO_LINKS included): only the long-range rows, thresholds and statistics.
+                             Refused (LDW_ERR_ARG) together with LDW_SCAN_SR_ONLY, which asks for no long-range table.
                              For inputs whose short-range table would not fit host memory (2000 x 500k SNPs in a 2.2 Mb
                              genome: 2.3e9 short-range links = 72 GB of columns) and for callers that only feed the
                              long-range links on (analyse_long_range_links, R/lr_analyser.R:72-108) */
@@ -205,6 +212,22 @@ LDW_API void ldw_mi_plan_destroy(ldw_mi_plan* plan);
  *   thr_out / prob_out : optional arrays of n_blocks doubles (NaN where the block had no LR branch)
  * Link lists are in reference order (blocks in make_blocks order; rows inside a block as
  * R/computePairwiseMI.R:306-310), LR rows being those that pass `MI >= disc_thresh` (:358).
+ *
+ * What each output flag returns, per table (n; host columns or NULL).  n_sr = stats_out->n_sr, n_kept =
+ * stats_out->n_lr_kept, border = the long-range rows within 1e-9 of their block's threshold.  thr_out, prob_out and the
+ * counts of stats_out do not depend on these flags.
+ *
+ *   output flags          sr_out           lr_out            borderline_out
+ *   (none)                n_sr, columns    n_kept, columns   border, columns
+ *   NO_D2H                n_sr, NULL       n_kept, NULL      0
+ *   NO_LINKS              n_sr, NULL       n_kept, NULL      0
+ *   LR_ONLY               0                n_kept, columns   border, columns
+ *   LR_ONLY | NO_D2H      0, NULL          n_kept, NULL      0
+ *   SR_ON_DEVICE          n_sr, NULL       n_kept, columns   border, columns
+ *
+ * ldw_group_mi_scan returns the same for the blocks of its local members (counts summed over them, columns merged into
+ * one table); with SR_ON_DEVICE and more than one local member no device holds the whole short-range table.  With SR_ONLY,
+ * n_kept and border are 0 under every output flag; SR_ONLY | LR_ONLY is refused with LDW_ERR_ARG before any device work.
  */
 LDW_API int ldw_mi_scan(ldw_mi_plan* plan, double g, double sr_dist, double lr_retain_links, double lr_links_approx,
                 int flags, int n_parts, int part, ldw_links* sr_out, ldw_links* lr_out, ldw_links* borderline_out,

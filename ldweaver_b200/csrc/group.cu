@@ -323,6 +323,7 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
                       double sr_dist, double lr_retain_links, double lr_links_approx, int flags, ldw_links* sr_out,
                       ldw_links* lr_out, ldw_links* borderline_out, double* thr_out, double* prob_out,
                       ldw_scan_stats* stats_out, double* t_plan_ms_out) {
+  LDW_TRY(validate_scan_flags(flags));  // on the caller's thread, before any device work
   if (!G) return set_error(LDW_ERR_ARG, "null group");
   if (G->n_snp <= 0) return set_error(LDW_ERR_ARG, "ldw_group_mi_scan: call ldw_group_load_codes first");
   if (!hdw || !pos || !paint) return set_error(LDW_ERR_ARG, "ldw_group_mi_scan: null argument");
@@ -366,10 +367,13 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
     sh.total_sr = total_sr;
     sh.h_sr = &G->h_sr;
     const bool want_host = !(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_NO_D2H));
+    // LDW_SCAN_SR_ON_DEVICE: every member keeps its short-range rows in its own device memory, so no host table is
+    // allocated or returned -- only the job's count (no member holds the whole table for ldw_sr_postprocess_dev either)
+    const bool sr_host = want_host && !(flags & LDW_SCAN_SR_ON_DEVICE);
     G->h_sr.n = 0; G->h_lr.n = 0; G->h_border.n = 0;
     const bool sr_rows = !(flags & (LDW_SCAN_NO_LINKS | LDW_SCAN_LR_ONLY));
     if (!sr_rows) total_sr = 0;
-    if (want_host) LDW_TRY(G->h_sr.ensure(total_sr));
+    if (sr_host) LDW_TRY(G->h_sr.ensure(total_sr));
     // ---- scan: one host thread per local device
     std::vector<ldw_links> lr(nl), bd(nl), srn(nl);
     std::vector<std::vector<double>> thr(nl, std::vector<double>(nblk, NAN)), prob(nl, std::vector<double>(nblk, NAN));
@@ -398,7 +402,7 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
       if (borderline_out) memset(borderline_out, 0, sizeof(*borderline_out));
       return 0;
     }
-    G->h_sr.n = total_sr;
+    if (sr_host) G->h_sr.n = total_sr;
     // long-range and borderline rows: every member's table is in make_blocks order and a block belongs to one member,
     // so the job's table is the members' runs of equal block id, taken in block order
     auto merge = [&](std::vector<ldw_links>& parts, HostLinks& dst) -> int {
@@ -430,7 +434,8 @@ int ldw_group_mi_scan(ldw_group* G, const double* hdw, const int32_t* pos, const
     };
     LDW_TRY(merge(lr, G->h_lr));
     LDW_TRY(merge(bd, G->h_border));
-    G->h_sr.fill(sr_out);
+    if (sr_host) G->h_sr.fill(sr_out);
+    else if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = total_sr; }
     G->h_lr.fill(lr_out);
     G->h_border.fill(borderline_out);
     return 0;

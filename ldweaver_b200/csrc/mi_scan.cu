@@ -724,6 +724,7 @@ RefineParams make_refine_params(const ldw_mi_plan* P, const BlockDev& D, const B
 }
 
 int validate_scan(const ldw_mi_plan* P, const ScanCfg& cfg) {
+  LDW_TRY(validate_scan_flags(cfg.flags));
   if (!(cfg.g > 0) || cfg.g != std::floor(cfg.g) || cfg.g > 9.0e15) return set_error(LDW_ERR_ARG, "genome length g=%g must be a positive integer", cfg.g);
   if (!(cfg.sr_dist >= 0)) return set_error(LDW_ERR_ARG, "sr_dist must be >= 0");
   if (!P->pos_sorted) return set_error(LDW_ERR_UNSUPPORTED, "POS must be non-decreasing (the short-range slot layout relies on it)");
@@ -859,6 +860,12 @@ int ldw_mi_scan(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links
 }
 
 }  // extern "C"
+
+int ldw::validate_scan_flags(int flags) {
+  if ((flags & LDW_SCAN_SR_ONLY) && (flags & LDW_SCAN_LR_ONLY))
+    return set_error(LDW_ERR_ARG, "LDW_SCAN_SR_ONLY and LDW_SCAN_LR_ONLY together ask for neither link table");
+  return 0;
+}
 
 // Sizes of every make_blocks block (pairs, short-range, long-range) on host threads: positions only, no device work.
 int ldw::mi_block_sizes(const ldw_mi_plan* P, double g, double sr_dist, int flags, std::vector<BlockSizes>& out) {
@@ -1410,7 +1417,8 @@ struct ScanRun {
       ctx->h_border.fill(borderline_out);
     }
     if (no_host) {
-      if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = total_sr; }
+      // LDW_SCAN_LR_ONLY: no short-range table, whatever else is asked (NO_LINKS still reports the short-range count)
+      if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = (cfg.flags & LDW_SCAN_LR_ONLY) ? 0 : total_sr; }
       if (lr_out) { memset(lr_out, 0, sizeof(*lr_out)); lr_out->n = (int64_t)n_kept; }
     } else {
       if (shared || !sr_to_host) { if (sr_out) { memset(sr_out, 0, sizeof(*sr_out)); sr_out->n = sr_rows ? total_sr : 0; } }
@@ -1515,6 +1523,7 @@ struct ScanRun {
 int ldw::mi_scan_impl(ldw_mi_plan* P, double g, double sr_dist, double lr_retain_links, double lr_links_approx, int flags,
                       int n_parts, int part, const ScanShared* shared, ldw_links* sr_out, ldw_links* lr_out,
                       ldw_links* borderline_out, double* thr_out, double* prob_out, ldw_scan_stats* stats_out) {
+  LDW_TRY(validate_scan_flags(flags));  // before any device work (and before the plan is looked at)
   if (!P) return set_error(LDW_ERR_ARG, "null plan");
   const auto t_entry = std::chrono::steady_clock::now();
   LDW_TRY(ctx_bind(P->ctx));

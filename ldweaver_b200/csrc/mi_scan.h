@@ -23,6 +23,8 @@ struct ScanShared {
 // (borrowed: it must outlive the plan).
 int mi_plan_create_impl(ldw_ctx* ctx, const uint8_t* codes, const uint8_t* codes_dev, int64_t n_snp, int64_t nseq,
                         const double* hdw, const int32_t* pos, const int32_t* paint, int64_t blk, ldw_mi_plan** out);
+// LDW_ERR_ARG for a combination of LDW_SCAN_* flags that asks for nothing (host only: callable before any device work)
+int validate_scan_flags(int flags);
 int mi_block_sizes(const ldw_mi_plan* P, double g, double sr_dist, int flags, std::vector<BlockSizes>& out);
 int64_t mi_plan_nblocks(const ldw_mi_plan* P);
 // owner[b] = part that scans make_blocks block b when the job is split n_parts ways (cost-based dealing)
