@@ -51,11 +51,7 @@ struct ldw_ctx {
   void (*scan_ws_free)(void*) = nullptr;
   // The short-range table the last scan on this context left in device memory (columns inside scan_ws; valid until the
   // next scan): what ldw_sr_postprocess_dev works on.  n < 0: none (no scan yet, a partial scan, or no rows materialised).
-  struct DevSr {
-    const int32_t *pos1 = nullptr, *pos2 = nullptr, *c1 = nullptr, *c2 = nullptr, *len = nullptr, *blk = nullptr;
-    const double* mi = nullptr;
-    int64_t n = -1;
-  } dev_sr;
+  ldw_links dev_sr = {-1};
 };
 
 namespace ldw {

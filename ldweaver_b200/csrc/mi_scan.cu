@@ -1427,11 +1427,8 @@ struct ScanRun {
       ctx->h_lr.fill(lr_out);
     }
     if (sr_rows && n_parts == 1) {  // the whole job's table is in this context's device memory, in reference order
-      ldw_ctx::DevSr& d = ctx->dev_sr;
-      d.pos1 = W->d_sr.pos1.as<int32_t>(); d.pos2 = W->d_sr.pos2.as<int32_t>(); d.c1 = W->d_sr.c1.as<int32_t>();
-      d.c2 = W->d_sr.c2.as<int32_t>(); d.len = W->d_sr.len.as<int32_t>(); d.blk = W->d_sr.blk.as<int32_t>();
-      d.mi = W->d_sr.mi.as<double>();
-      d.n = total_sr;
+      W->d_sr.fill(&ctx->dev_sr);
+      ctx->dev_sr.n = total_sr;
     }
     for (size_t b = 0; b < blocks.size(); b++) {
       if (sel[b].skip || sel[b].n_lr == 0 || sr_only) continue;

@@ -19,20 +19,25 @@
 //   7. cub::DeviceSelect::Flagged per cluster: the links above the fit in scan order (the reference's row order)
 //   8. sr_srp_kernel           srp_max = -pbeta(d, a, b, lower = F, log = T) in fp64 (continued fraction, :453), and the smallest
 //                              MI among the same-cluster links with srp_max > cutoff
-//   9. sr_keep_kernel + select + sr_gather_kernel: ONLY the rows sr_links_red (srp_max > cutoff, :494) and
+//   9. select on the dup flags: row ids, srp_max and the compared columns of the (few) cross-cluster links come to the
+//                              host, which keeps them once each (:474-483; shared code)
+//  10. sr_keep_kernel + select: row ids and srp_max of ONLY the same-cluster rows sr_links_red (srp_max > cutoff, :494) and
 //                              sr_links_ARACNE_check (MI >= min(sr_links_red$MI), :495) need -- a few 10^5 of the 4.5 x 10^6
-//                              links above the fit at 616 x 100k -- and the (few) cross-cluster links, which the host keeps
-//                              once each (:474-483; shared code), come to the host
+//                              links above the fit at 616 x 100k
+//  11. gather_kernel per column: the link columns of those df rows, by row id, in df order
+// The membership filter, the residual lookup and the beta tail are the host implementation's own (sr_stats.cuh).
 #include <cub/cub.cuh>
 #include <thrust/iterator/counting_iterator.h>
 
 #include <chrono>
 #include <cmath>
 #include <memory>
+#include <numeric>
 
 #include "../../include/ldw.h"
 #include "ctx.h"
 #include "post_host.h"
+#include "sr_stats.cuh"
 
 using namespace ldw;
 
@@ -40,26 +45,10 @@ namespace {
 
 constexpr int MAXC = 64;  // clusters handled on the device path (cds_var$nclust is 2-3 in practice)
 
-struct SrCols {
-  const int32_t *c1, *c2, *len;
-  const double* mi;
-  int64_t n;
-};
-
-// clusters a link is listed under (0 = none): clust1 and, if different, clust2; only 0 < len < sr_dist
-__device__ __forceinline__ bool sr_member(const SrCols& T, int64_t i, double sr_dist, int nclust, int& ca, int& cb, int& l) {
-  l = T.len[i];
-  if (!(l > 0 && (double)l < sr_dist)) return false;
-  ca = T.c1[i]; cb = T.c2[i];
-  if (ca < 1 || ca > nclust) ca = 0;
-  if (cb < 1 || cb > nclust || cb == ca) cb = 0;
-  return (ca | cb) != 0;
-}
-
-__global__ void sr_group_count_kernel(SrCols T, double sr_dist, int nclust, int64_t nl, uint32_t* gcount) {
+__global__ void sr_group_count_kernel(ldw_links T, double sr_dist, int nclust, int64_t nl, uint32_t* gcount) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < T.n; i += (int64_t)gridDim.x * blockDim.x) {
     int ca, cb, l;
-    if (!sr_member(T, i, sr_dist, nclust, ca, cb, l)) continue;
+    if (!ldwpost::member(T, i, sr_dist, nclust, ca, cb, l)) continue;
     if (ca) atomicAdd(&gcount[(int64_t)(ca - 1) * nl + l], 1u);
     if (cb) atomicAdd(&gcount[(int64_t)(cb - 1) * nl + l], 1u);
   }
@@ -70,12 +59,12 @@ __global__ void u32_to_i64_kernel(const uint32_t* in, int64_t n, int64_t* out) {
   if (i < n) out[i] = in[i];
 }
 
-__global__ void sr_group_scatter_kernel(SrCols T, double sr_dist, int nclust, int64_t nl, const int64_t* goff, unsigned long long* cursor,
+__global__ void sr_group_scatter_kernel(ldw_links T, double sr_dist, int nclust, int64_t nl, const int64_t* goff, unsigned long long* cursor,
                                         double* keys) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < T.n; i += (int64_t)gridDim.x * blockDim.x) {
     int ca, cb, l;
-    if (!sr_member(T, i, sr_dist, nclust, ca, cb, l)) continue;
-    const double v = T.mi[i];
+    if (!ldwpost::member(T, i, sr_dist, nclust, ca, cb, l)) continue;
+    const double v = T.MI[i];
     if (ca) { const int64_t g = (int64_t)(ca - 1) * nl + l; keys[goff[g] + (int64_t)atomicAdd(&cursor[g], 1ull)] = v; }
     if (cb) { const int64_t g = (int64_t)(cb - 1) * nl + l; keys[goff[g] + (int64_t)atomicAdd(&cursor[g], 1ull)] = v; }
   }
@@ -108,16 +97,10 @@ struct FitTab {           // fitted decay per cluster as the reference subscript
   int nclust;
 };
 
-__device__ __forceinline__ bool sr_residual(const FitTab& F, int c, int l, double mi, double& d) {
-  if ((int64_t)l > F.off[c] - F.off[c - 1]) return false;  // NA in R: drops out of which(diff > 0)
-  d = mi - F.val[F.off[c - 1] + l - 1];
-  return d > 0;
-}
-
 constexpr int RES_THREADS = 256;
 // Each block owns one contiguous piece of the table; its partial sums are reduced in a fixed order (strided per-thread
 // accumulation, then a shared-memory tree), so the totals do not depend on scheduling.
-__global__ void __launch_bounds__(RES_THREADS) sr_residual_kernel(SrCols T, double sr_dist, FitTab F, int64_t piece, uint8_t* flags /*[nclust][N]*/,
+__global__ void __launch_bounds__(RES_THREADS) sr_residual_kernel(ldw_links T, double sr_dist, FitTab F, int64_t piece, uint8_t* flags /*[nclust][N]*/,
                                                                   double* part /*[blocks][nclust][5]*/, uint32_t* bad) {
   __shared__ double sh[RES_THREADS];
   const int64_t lo = (int64_t)blockIdx.x * piece, hi = min(T.n, lo + piece);
@@ -126,9 +109,9 @@ __global__ void __launch_bounds__(RES_THREADS) sr_residual_kernel(SrCols T, doub
     for (int64_t i = lo + threadIdx.x; i < hi; i += RES_THREADS) {
       int ca, cb, l;
       uint8_t f = 0;
-      if (sr_member(T, i, sr_dist, F.nclust, ca, cb, l) && (ca == c || cb == c)) {
+      if (ldwpost::member(T, i, sr_dist, F.nclust, ca, cb, l) && (ca == c || cb == c)) {
         double d;
-        if (sr_residual(F, c, l, T.mi[i], d)) {
+        if (ldwpost::residual(F.val, F.off, c, l, T.MI[i], d)) {
           f = 1;
           if (d > 1) atomicMax(bad, (uint32_t)c);
           acc[0] += 1.0; acc[1] += log(d); acc[2] += log1p(-d); acc[3] += d; acc[4] += d * d;
@@ -149,45 +132,6 @@ __global__ void __launch_bounds__(RES_THREADS) sr_residual_kernel(SrCols T, doub
   }
 }
 
-// ---- log of the regularised incomplete beta function (continued fraction, modified Lentz): post_host.cpp:log_ibeta_cf ----
-__device__ double d_log_ibeta_cf(double a, double b, double x, double logx, double log1mx, double lbeta) {
-  const double tiny = 1e-300, eps = 1e-16;
-  const double qab = a + b, qap = a + 1.0, qam = a - 1.0;
-  double c = 1.0, d = 1.0 - qab * x / qap;
-  if (fabs(d) < tiny) d = tiny;
-  d = 1.0 / d;
-  double h = d;
-  for (int m = 1; m <= 10000; m++) {
-    const double m2 = 2.0 * m;
-    double aa = m * (b - m) * x / ((qam + m2) * (a + m2));
-    d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
-    c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
-    d = 1.0 / d;
-    h *= d * c;
-    aa = -(a + m) * (qab + m) * x / ((a + m2) * (qap + m2));
-    d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
-    c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
-    d = 1.0 / d;
-    const double del = d * c;
-    h *= del;
-    if (fabs(del - 1.0) < eps) break;
-  }
-  return a * logx + b * log1mx - lbeta - log(a) + log(h);
-}
-
-__device__ double d_neg_log_upper_beta(double x, double a, double b, double lbeta) {
-  const double logx = log(x), log1mx = log1p(-x);
-  const double y = 1.0 - x;
-  if (y < (b + 1.0) / (a + b + 2.0)) return -d_log_ibeta_cf(b, a, y, log1mx, logx, lbeta);
-  const double lp = d_log_ibeta_cf(a, b, x, logx, log1mx, lbeta);
-  return -log1p(-exp(lp));
-}
-
-struct FullCols {
-  const int32_t *pos1, *pos2, *c1, *c2, *len, *blk;
-  const double* mi;
-};
-
 // order-preserving 64-bit key of a double (for atomicMin on MI values, which may be negative)
 __device__ __forceinline__ unsigned long long dbl_key(double v) {
   unsigned long long b = (unsigned long long)__double_as_longlong(v);
@@ -196,47 +140,48 @@ __device__ __forceinline__ unsigned long long dbl_key(double v) {
 
 // srp_max of the links above the fit of cluster c (rows[k]); dup[k] = the link joins two clusters (it is listed under both
 // and de-duplicated on the host); *min_red_key = smallest MI among the same-cluster links that pass the cut-off.
-__global__ void sr_srp_kernel(FullCols T, FitTab F, int c, double a, double b, double lbeta, double cutoff, const int64_t* rows, int64_t n,
+__global__ void sr_srp_kernel(ldw_links T, FitTab F, int c, double a, double b, double lbeta, double cutoff, const int64_t* rows, int64_t n,
                               double* srp, uint8_t* dup, unsigned long long* min_red_key) {
   int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n) return;
   const int64_t i = rows[k];
-  const double mi = T.mi[i];
-  const double d = mi - F.val[F.off[c - 1] + T.len[i] - 1];
-  const double v = d < 1.0 ? d_neg_log_upper_beta(d, a, b, lbeta) : INFINITY;
+  const double mi = T.MI[i];
+  const double d = mi - ldwpost::fit_at(F.val, F.off, c, T.len[i]);
+  const double v = d < 1.0 ? ldwpost::neg_log_upper_beta(d, a, b, lbeta) : INFINITY;
   srp[k] = v;
-  const bool is_dup = T.c1[i] != T.c2[i];
+  const bool is_dup = T.clust1[i] != T.clust2[i];
   dup[k] = is_dup ? 1 : 0;
   if (!is_dup && v > cutoff) atomicMin(min_red_key, dbl_key(mi));  // NaN compares false: dropped as in :458
 }
 
-// which rows of the cluster's list travel to the host: every cross-cluster link (few; de-duplicated there), and the
-// same-cluster links that are in sr_links_red (srp_max > cutoff) or in sr_links_ARACNE_check (MI >= min_mi)
-__global__ void sr_keep_kernel(FullCols T, const int64_t* rows, const double* srp, const uint8_t* dup, int64_t n, double cutoff, double min_mi,
-                               int phase, uint8_t* keep) {
+// which same-cluster rows of the cluster's list travel to the host: those in sr_links_red (srp_max > cutoff) or in
+// sr_links_ARACNE_check (MI >= min_mi)
+__global__ void sr_keep_kernel(ldw_links T, const int64_t* rows, const double* srp, const uint8_t* dup, int64_t n, double cutoff, double min_mi,
+                               uint8_t* keep) {
   int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= n) return;
   const double v = srp[k];
-  bool kp;
-  if (phase == 0) kp = dup[k] != 0;
-  else kp = !dup[k] && !isnan(v) && (v > cutoff || T.mi[rows[k]] >= min_mi);
-  keep[k] = kp ? 1 : 0;
+  keep[k] = (!dup[k] && !isnan(v) && (v > cutoff || T.MI[rows[k]] >= min_mi)) ? 1 : 0;
 }
 
-__global__ void sr_gather_kernel(FullCols T, const int64_t* rows, const double* srp, const int64_t* pick, int64_t n, int64_t* o_row, double* o_srp,
-                                 int32_t* o_pos1, int32_t* o_pos2, int32_t* o_c1, int32_t* o_c2, int32_t* o_len, int32_t* o_blk, double* o_mi) {
+template <class T>
+__global__ void gather_kernel(const T* src, const int64_t* idx, int64_t n, T* dst) {
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n) return;
-  const int64_t k = pick[t], i = rows[k];
-  o_row[t] = i; o_srp[t] = srp[k];
-  o_pos1[t] = T.pos1[i]; o_pos2[t] = T.pos2[i]; o_c1[t] = T.c1[i]; o_c2[t] = T.c2[i]; o_len[t] = T.len[i]; o_blk[t] = T.blk[i]; o_mi[t] = T.mi[i];
+  if (t < n) dst[t] = src[idx[t]];
 }
 
-__global__ void max_len_kernel(SrCols T, double sr_dist, int nclust, int* out) {
+// dst[t] = src[idx[t]], t < n, elements of el (4 or 8) bytes
+void gather(const void* src, size_t el, const int64_t* idx, int64_t n, void* dst, cudaStream_t st) {
+  const unsigned nb = (unsigned)((n + 255) / 256);
+  if (el == 8) gather_kernel<<<nb, 256, 0, st>>>(static_cast<const uint64_t*>(src), idx, n, static_cast<uint64_t*>(dst));
+  else gather_kernel<<<nb, 256, 0, st>>>(static_cast<const uint32_t*>(src), idx, n, static_cast<uint32_t*>(dst));
+}
+
+__global__ void max_len_kernel(ldw_links T, double sr_dist, int nclust, int* out) {
   int m = 0;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < T.n; i += (int64_t)gridDim.x * blockDim.x) {
     int ca, cb, l;
-    if (sr_member(T, i, sr_dist, nclust, ca, cb, l)) m = max(m, l);
+    if (ldwpost::member(T, i, sr_dist, nclust, ca, cb, l)) m = max(m, l);
   }
   for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
   if ((threadIdx.x & 31) == 0 && m) atomicMax(out, m);
@@ -251,13 +196,12 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
     if (df_rows_out) memset(df_rows_out, 0, sizeof(*df_rows_out));
     LDW_TRY(ctx_bind(ctx));
     if (nclust < 1 || nclust > MAXC) return set_error(LDW_ERR_UNSUPPORTED, "ldw_sr_postprocess_dev: nclust must be in 1..%d", MAXC);
-    const ldw_ctx::DevSr& D = ctx->dev_sr;
-    if (D.n < 0) return set_error(LDW_ERR_ARG, "ldw_sr_postprocess_dev: no short-range table on the device (run ldw_mi_scan over the whole job, "
+    const ldw_links& T = ctx->dev_sr;
+    if (T.n < 0) return set_error(LDW_ERR_ARG, "ldw_sr_postprocess_dev: no short-range table on the device (run ldw_mi_scan over the whole job, "
                                                 "n_parts = 1, without LDW_SCAN_NO_LINKS / LDW_SCAN_LR_ONLY, first)");
-    const int64_t N = D.n;
+    const int64_t N = T.n;
     if (N > 0x7fffffffLL) return set_error(LDW_ERR_UNSUPPORTED, "ldw_sr_postprocess_dev: more than 2^31 short-range links");
     cudaStream_t st = ctx->stream;
-    SrCols T{D.c1, D.c2, D.len, D.mi, N};
     std::unique_ptr<ldwpost::SrPostPriv> S(new ldwpost::SrPostPriv());
     S->fit_off.assign(1, 0);
     const int nb_stream = ctx->num_sms * 8;
@@ -272,10 +216,9 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
     };
 
     // ---- groups: (cluster, length) ----
-    int32_t maxlen = 0;
-    if (sr_dist <= (double)(1 << 18)) {
-      maxlen = (int32_t)std::max(0.0, ceil(sr_dist) - 1.0);
-    } else {
+    int32_t maxlen = ldwpost::max_len_bound(sr_dist);
+    if (maxlen < 0) {
+      maxlen = 0;
       DevBuf d_m;
       LDW_TRY(d_m.alloc(4));
       LDW_CUDA(cudaMemsetAsync(d_m.p, 0, 4, st));
@@ -310,9 +253,7 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
     LDW_CUDA(cudaStreamSynchronize(st));
     const int64_t E = goff[G];
     lap("group histogram + offsets");
-    for (int32_t c = 1; c <= nclust; c++)
-      if (goff[(int64_t)c * nl] == goff[(int64_t)(c - 1) * nl])
-        return set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d holds no short-range link with 0 < len < sr_dist", (int)c);
+    LDW_TRY(ldwpost::check_groups(goff, nclust, nl));
     // ---- per-group 95th percentiles ----
     std::vector<double> gq_all((size_t)G);
     {
@@ -365,17 +306,27 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
     LDW_CUDA(cudaMemcpyAsync(part.data(), d_part.p, part.size() * 8, cudaMemcpyDeviceToHost, st));
     LDW_CUDA(cudaMemcpyAsync(&bad, d_bad.p, 4, cudaMemcpyDeviceToHost, st));
     LDW_CUDA(cudaStreamSynchronize(st));
-    if (bad) return set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d: values must be in [0-1] to fit a beta distribution", (int)bad);
+    LDW_TRY(ldwpost::check_residuals((int)bad));
     lap("residual flags + sums");
 
-    FullCols FT{D.pos1, D.pos2, D.c1, D.c2, D.len, D.blk, D.mi};
     // Per cluster: the links above the fit in scan order, their srp_max, the smallest MI of those that pass the cut-off.
     struct PerC { DevBuf rows, srp, dup; int64_t npos = 0; };
     std::vector<PerC> pc((size_t)nclust + 1);
-    DevBuf d_tmp, d_nsel, d_minkey, d_keep, d_pick;
+    DevBuf d_tmp, d_nsel, d_minkey, d_keep, d_pick, d_row, d_col;
     LDW_TRY(d_nsel.alloc(8));
     LDW_TRY(d_minkey.alloc(8));
     LDW_CUDA(cudaMemsetAsync(d_minkey.p, 0xFF, 8, st));
+    // out[0 .. m) = the positions of the set flags among n, in order
+    auto select_flagged = [&](const uint8_t* flags, int64_t n, int64_t* out, int64_t& m) -> int {
+      thrust::counting_iterator<int64_t> it(0);
+      size_t tb = 0;
+      cub::DeviceSelect::Flagged(nullptr, tb, it, flags, out, d_nsel.as<int64_t>(), (int)n, st);
+      LDW_TRY(d_tmp.ensure(tb));
+      LDW_CUDA(cub::DeviceSelect::Flagged(d_tmp.p, tb, it, flags, out, d_nsel.as<int64_t>(), (int)n, st));
+      LDW_CUDA(cudaMemcpyAsync(&m, d_nsel.p, 8, cudaMemcpyDeviceToHost, st));
+      LDW_CUDA(cudaStreamSynchronize(st));
+      return 0;
+    };
     for (int32_t c = 1; c <= nclust; c++) {
       long double cnt = 0, s1 = 0, s2 = 0, sm = 0, sq = 0;
       for (int64_t k = 0; k < nblocks; k++) {
@@ -383,7 +334,7 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
         cnt += p[0]; s1 += p[1]; s2 += p[2]; sm += p[3]; sq += p[4];
       }
       const int64_t npos = (int64_t)llroundl(cnt);
-      if (npos < 2) return set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d has fewer than two links above the fitted decay", (int)c);
+      LDW_TRY(ldwpost::check_npos(c, npos));
       const double mean = (double)(sm / (long double)npos);
       const double v = (double)((sq - (long double)npos * (long double)mean * (long double)mean) / (long double)npos);  // biased variance
       double par[2];
@@ -394,19 +345,10 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
       LDW_TRY(P.rows.alloc((size_t)npos * 8));
       LDW_TRY(P.srp.alloc((size_t)npos * 8));
       LDW_TRY(P.dup.alloc((size_t)npos));
-      {
-        thrust::counting_iterator<int64_t> it(0);
-        size_t tb = 0;
-        cub::DeviceSelect::Flagged(nullptr, tb, it, d_flags.as<uint8_t>() + (size_t)(c - 1) * N, P.rows.as<int64_t>(), d_nsel.as<int64_t>(), (int)N, st);
-        LDW_TRY(d_tmp.ensure(tb));
-        LDW_CUDA(cub::DeviceSelect::Flagged(d_tmp.p, tb, it, d_flags.as<uint8_t>() + (size_t)(c - 1) * N, P.rows.as<int64_t>(),
-                                            d_nsel.as<int64_t>(), (int)N, st));
-      }
       int64_t nsel = 0;
-      LDW_CUDA(cudaMemcpyAsync(&nsel, d_nsel.p, 8, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaStreamSynchronize(st));
+      LDW_TRY(select_flagged(d_flags.as<uint8_t>() + (size_t)(c - 1) * N, N, P.rows.as<int64_t>(), nsel));
       if (nsel != npos) return set_error(LDW_ERR_INTERNAL, "ldw_sr_postprocess_dev: %lld flagged links but %lld counted", (long long)nsel, (long long)npos);
-      sr_srp_kernel<<<(unsigned)((npos + 127) / 128), 128, 0, st>>>(FT, F, c, par[0], par[1], lbeta, srp_cutoff, P.rows.as<int64_t>(), npos,
+      sr_srp_kernel<<<(unsigned)((npos + 127) / 128), 128, 0, st>>>(T, F, c, par[0], par[1], lbeta, srp_cutoff, P.rows.as<int64_t>(), npos,
                                                                    P.srp.as<double>(), P.dup.as<uint8_t>(), d_minkey.as<unsigned long long>());
       LDW_CUDA(cudaGetLastError());
     }
@@ -414,69 +356,64 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
     // Only what sr_links_red / sr_links_ARACNE_check need comes to the host (sr_links_df itself -- every link above the fit,
     // 4.5e6 rows at 616 x 100k -- stays on the device): first the cross-cluster links, whose de-duplication decides which of
     // them are in sr_links_red and therefore min(sr_links_red$MI); then the same-cluster rows of the two sets.
-    struct Got { std::vector<int64_t> row; std::vector<double> srp, mi; std::vector<int32_t> pos1, pos2, c1, c2, len, blk; };
-    auto fetch = [&](int32_t c, int phase, double min_mi, Got& G) -> int {
+    // pick: rows and srp_max of the entries of cluster c's list whose flag is set, in scan order.
+    auto pick = [&](int32_t c, const uint8_t* flags, std::vector<int64_t>& row, std::vector<double>& srp) -> int {
       PerC& P = pc[c];
-      const int64_t npos = P.npos;
-      LDW_TRY(d_keep.ensure((size_t)npos));
-      LDW_TRY(d_pick.ensure((size_t)npos * 8));
-      sr_keep_kernel<<<(unsigned)((npos + 255) / 256), 256, 0, st>>>(FT, P.rows.as<int64_t>(), P.srp.as<double>(), P.dup.as<uint8_t>(), npos, srp_cutoff,
-                                                                    min_mi, phase, d_keep.as<uint8_t>());
-      thrust::counting_iterator<int64_t> it(0);
-      size_t tb = 0;
-      cub::DeviceSelect::Flagged(nullptr, tb, it, d_keep.as<uint8_t>(), d_pick.as<int64_t>(), d_nsel.as<int64_t>(), (int)npos, st);
-      LDW_TRY(d_tmp.ensure(tb));
-      LDW_CUDA(cub::DeviceSelect::Flagged(d_tmp.p, tb, it, d_keep.as<uint8_t>(), d_pick.as<int64_t>(), d_nsel.as<int64_t>(), (int)npos, st));
       int64_t m = 0;
-      LDW_CUDA(cudaMemcpyAsync(&m, d_nsel.p, 8, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaStreamSynchronize(st));
-      G.row.resize((size_t)m); G.srp.resize((size_t)m); G.mi.resize((size_t)m);
-      for (auto* v32 : {&G.pos1, &G.pos2, &G.c1, &G.c2, &G.len, &G.blk}) v32->resize((size_t)m);
+      LDW_TRY(d_pick.ensure((size_t)P.npos * 8));
+      LDW_TRY(select_flagged(flags, P.npos, d_pick.as<int64_t>(), m));
+      row.resize((size_t)m);
+      srp.resize((size_t)m);
       if (m == 0) return 0;
-      DevBuf o_row, o_srp, o1, o2, o3, o4, o5, o6, o7;
-      LDW_TRY(o_row.alloc((size_t)m * 8)); LDW_TRY(o_srp.alloc((size_t)m * 8)); LDW_TRY(o7.alloc((size_t)m * 8));
-      LDW_TRY(o1.alloc((size_t)m * 4)); LDW_TRY(o2.alloc((size_t)m * 4)); LDW_TRY(o3.alloc((size_t)m * 4));
-      LDW_TRY(o4.alloc((size_t)m * 4)); LDW_TRY(o5.alloc((size_t)m * 4)); LDW_TRY(o6.alloc((size_t)m * 4));
-      sr_gather_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(FT, P.rows.as<int64_t>(), P.srp.as<double>(), d_pick.as<int64_t>(), m, o_row.as<int64_t>(),
-                                                                   o_srp.as<double>(), o1.as<int32_t>(), o2.as<int32_t>(), o3.as<int32_t>(), o4.as<int32_t>(),
-                                                                   o5.as<int32_t>(), o6.as<int32_t>(), o7.as<double>());
+      LDW_TRY(d_row.ensure((size_t)m * 8));
+      LDW_TRY(d_col.ensure((size_t)m * 8));
+      gather(P.rows.p, 8, d_pick.as<int64_t>(), m, d_row.p, st);
+      gather(P.srp.p, 8, d_pick.as<int64_t>(), m, d_col.p, st);
       LDW_CUDA(cudaGetLastError());
-      LDW_CUDA(cudaMemcpyAsync(G.row.data(), o_row.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.srp.data(), o_srp.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.mi.data(), o7.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.pos1.data(), o1.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.pos2.data(), o2.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.c1.data(), o3.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.c2.data(), o4.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.len.data(), o5.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
-      LDW_CUDA(cudaMemcpyAsync(G.blk.data(), o6.p, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
+      LDW_CUDA(cudaMemcpyAsync(row.data(), d_row.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
+      LDW_CUDA(cudaMemcpyAsync(srp.data(), d_col.p, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
       LDW_CUDA(cudaStreamSynchronize(st));
       return 0;
     };
-    auto append = [&](const Got& G, int64_t t) -> int64_t {  // one row into the gathered table; returns its position
-      S->g_pos1.push_back(G.pos1[t]); S->g_pos2.push_back(G.pos2[t]); S->g_c1.push_back(G.c1[t]); S->g_c2.push_back(G.c2[t]);
-      S->g_len.push_back(G.len[t]); S->g_blk.push_back(G.blk[t]); S->g_mi.push_back(G.mi[t]);
-      return (int64_t)S->g_mi.size() - 1;
+    // fetch: the link columns of table rows `row` into o, in that order (all, or only those the de-duplication compares).
+    auto fetch = [&](const std::vector<int64_t>& row, ldwpost::HostCols& o, bool all) -> int {
+      const int64_t m = (int64_t)row.size();
+      LDW_TRY(o.ensure(m));
+      o.n = m;
+      if (m == 0) return 0;
+      LDW_TRY(d_row.ensure((size_t)m * 8));
+      LDW_TRY(d_col.ensure((size_t)m * 8));
+      LDW_CUDA(cudaMemcpyAsync(d_row.p, row.data(), (size_t)m * 8, cudaMemcpyHostToDevice, st));
+      for (int k = 0; k < ldwpost::HostCols::NCOL; k++) {
+        if (!all && &o.col(k) == &o.blk) continue;
+        const size_t el = ldwpost::HostCols::elem(k);
+        gather(ldwpost::HostCols::abi_col(T, k), el, d_row.as<int64_t>(), m, d_col.p, st);
+        LDW_CUDA(cudaGetLastError());
+        LDW_CUDA(cudaMemcpyAsync(o.col(k).p.get(), d_col.p, (size_t)m * el, cudaMemcpyDeviceToHost, st));
+      }
+      LDW_CUDA(cudaStreamSynchronize(st));
+      return 0;
     };
     // ---- phase 0: cross-cluster links -> de-duplicated (:474-483) ----
-    std::vector<int64_t> dup_row, dup_at, dup_keep_row, dup_keep_at;
-    std::vector<int32_t> dup_c, dup_keep_c;
-    std::vector<double> dup_srp, dup_keep_srp;
+    std::vector<int64_t> dup_row;
+    std::vector<int32_t> dup_c;
+    std::vector<double> dup_srp;
     for (int32_t c = 1; c <= nclust; c++) {
-      Got G;
-      LDW_TRY(fetch(c, 0, 0.0, G));
-      for (size_t t = 0; t < G.row.size(); t++) {
-        if (std::isnan(G.srp[t])) continue;  // :458
-        dup_row.push_back(G.row[t]); dup_at.push_back(append(G, (int64_t)t)); dup_c.push_back(c); dup_srp.push_back(G.srp[t]);
+      std::vector<int64_t> row;
+      std::vector<double> srp;
+      LDW_TRY(pick(c, pc[c].dup.as<uint8_t>(), row, srp));
+      for (size_t t = 0; t < row.size(); t++) {
+        if (std::isnan(srp[t])) continue;  // :458
+        dup_row.push_back(row[t]); dup_c.push_back(c); dup_srp.push_back(srp[t]);
       }
     }
-    {
-      ldwpost::SrPostPriv tmp;  // run the shared de-duplication on the cross-cluster links alone
-      ldwpost::LinkCols cols{S->g_pos1.data(), S->g_pos2.data(), S->g_c1.data(), S->g_c2.data(), S->g_len.data(), S->g_mi.data()};
-      std::vector<int64_t> at;
-      ldwpost::dedup_and_select(tmp, cols, dup_row, dup_at, dup_c, dup_srp, at, INFINITY);
-      dup_keep_row = tmp.row; dup_keep_c = tmp.clust_c; dup_keep_srp = tmp.srp; dup_keep_at = at;
-    }
+    ldwpost::HostCols dup_cols;
+    LDW_TRY(fetch(dup_row, dup_cols, false));
+    ldw_links dup_tab;
+    dup_cols.fill(&dup_tab);
+    std::vector<int64_t> dup_at(dup_row.size());
+    std::iota(dup_at.begin(), dup_at.end(), 0);
+    const std::vector<int64_t> win = ldwpost::dedup(dup_tab, dup_at, dup_srp);
     unsigned long long minkey = ~0ull;
     LDW_CUDA(cudaMemcpyAsync(&minkey, d_minkey.p, 8, cudaMemcpyDeviceToHost, st));
     LDW_CUDA(cudaStreamSynchronize(st));
@@ -485,49 +422,38 @@ extern "C" int ldw_sr_postprocess_dev(ldw_ctx* ctx, int32_t nclust, double sr_di
       const unsigned long long bts = (minkey >> 63) ? (minkey & 0x7FFFFFFFFFFFFFFFull) : ~minkey;
       memcpy(&min_mi, &bts, 8);
     }
-    for (size_t k = 0; k < dup_keep_row.size(); k++)
-      if (dup_keep_srp[k] > srp_cutoff) min_mi = std::min(min_mi, S->g_mi[(size_t)dup_keep_at[k]]);
+    for (int64_t k : win)
+      if (dup_srp[k] > srp_cutoff) min_mi = std::min(min_mi, dup_tab.MI[k]);
     lap("cross-cluster links + min MI");
     // ---- phase 1: same-cluster rows of sr_links_red / sr_links_ARACNE_check, cluster by cluster in scan order ----
-    std::vector<int64_t> df_at;
     for (int32_t c = 1; c <= nclust; c++) {
-      Got G;
-      LDW_TRY(fetch(c, 1, min_mi, G));
-      for (size_t t = 0; t < G.row.size(); t++) {
-        S->row.push_back(G.row[t]); S->clust_c.push_back(c); S->srp.push_back(G.srp[t]);
-        df_at.push_back(append(G, (int64_t)t));
-      }
+      PerC& P = pc[c];
+      LDW_TRY(d_keep.ensure((size_t)P.npos));
+      sr_keep_kernel<<<(unsigned)((P.npos + 255) / 256), 256, 0, st>>>(T, P.rows.as<int64_t>(), P.srp.as<double>(), P.dup.as<uint8_t>(), P.npos,
+                                                                       srp_cutoff, min_mi, d_keep.as<uint8_t>());
+      LDW_CUDA(cudaGetLastError());
+      std::vector<int64_t> row;
+      std::vector<double> srp;
+      LDW_TRY(pick(c, d_keep.as<uint8_t>(), row, srp));
+      S->row.insert(S->row.end(), row.begin(), row.end());
+      S->clust_c.insert(S->clust_c.end(), row.size(), c);
+      S->srp.insert(S->srp.end(), srp.begin(), srp.end());
     }
-    for (size_t k = 0; k < dup_keep_row.size(); k++) {  // the de-duplicated cross-cluster links follow (:483), those in either set
-      const double mi = S->g_mi[(size_t)dup_keep_at[k]];
-      if (!(dup_keep_srp[k] > srp_cutoff || mi >= min_mi)) continue;
-      S->row.push_back(dup_keep_row[k]); S->clust_c.push_back(dup_keep_c[k]); S->srp.push_back(dup_keep_srp[k]);
-      df_at.push_back(dup_keep_at[k]);
+    for (int64_t k : win) {  // the de-duplicated cross-cluster links follow (:483), those in either set
+      if (!(dup_srp[k] > srp_cutoff || dup_tab.MI[k] >= min_mi)) continue;
+      S->row.push_back(dup_row[k]); S->clust_c.push_back(dup_c[k]); S->srp.push_back(dup_srp[k]);
     }
+    LDW_TRY(fetch(S->row, S->df, true));
     lap("rows of red / check sets");
     const int64_t ndf = (int64_t)S->row.size();
+    const double* df_mi = S->df.mi.as<double>();
     for (int64_t i = 0; i < ndf; i++) {
       if (S->srp[(size_t)i] > srp_cutoff) S->red.push_back(i);
-      if (S->g_mi[(size_t)df_at[(size_t)i]] >= min_mi) S->chk.push_back(i);
-    }
-    {  // the gathered columns in df order (the gathered table also holds the losing copies of cross-cluster links)
-      std::vector<int32_t> a1(ndf), a2(ndf), a3(ndf), a4(ndf), a5(ndf), a6(ndf);
-      std::vector<double> a7(ndf);
-      for (int64_t k = 0; k < ndf; k++) {
-        const int64_t at = df_at[(size_t)k];
-        a1[k] = S->g_pos1[at]; a2[k] = S->g_pos2[at]; a3[k] = S->g_c1[at]; a4[k] = S->g_c2[at]; a5[k] = S->g_len[at]; a6[k] = S->g_blk[at];
-        a7[k] = S->g_mi[at];
-      }
-      S->g_pos1.swap(a1); S->g_pos2.swap(a2); S->g_c1.swap(a3); S->g_c2.swap(a4); S->g_len.swap(a5); S->g_blk.swap(a6); S->g_mi.swap(a7);
+      if (df_mi[i] >= min_mi) S->chk.push_back(i);
     }
     lap("red / chk + reorder (host)");
     ldwpost::publish(*S, nclust, out);
-    if (df_rows_out) {
-      df_rows_out->n = out->n_df;
-      df_rows_out->pos1 = S->g_pos1.data(); df_rows_out->pos2 = S->g_pos2.data(); df_rows_out->clust1 = S->g_c1.data();
-      df_rows_out->clust2 = S->g_c2.data(); df_rows_out->len = S->g_len.data(); df_rows_out->MI = S->g_mi.data();
-      df_rows_out->block = S->g_blk.data();
-    }
+    S->df.fill(df_rows_out);
     out->priv = S.release();
     return 0;
   });

@@ -35,6 +35,7 @@
 
 #include "host_util.h"
 #include "post_host.h"
+#include "sr_stats.cuh"
 #include "../../include/ldw.h"
 
 using ldwpost::SrPostPriv;
@@ -167,9 +168,7 @@ struct BetaNll {
   double operator()(const double* p) const {
     const double a = p[0], b = p[1];
     if (!(a > 0 && b > 0)) return NAN;  // dbeta gives NaN there; nmmin replaces a non-finite value by `big`
-    int sg;
-    const double lbeta = lgamma_r(a, &sg) + lgamma_r(b, &sg) - lgamma_r(a + b, &sg);
-    return -((a - 1) * s1 + (b - 1) * s2 - n * lbeta);
+    return -((a - 1) * s1 + (b - 1) * s2 - n * ldwpost::lbeta_fn(a, b));
   }
 };
 
@@ -280,42 +279,6 @@ int nmmin2(const Fn& fn, const double start[2], double xout[2], double* fmin, in
   return fail;
 }
 
-// ---- log of the regularised incomplete beta function, continued fraction evaluated with the modified Lentz scheme ----
-// log I_x(a, b) given log(x) and log(1 - x); converges fast for x < (a + 1) / (a + b + 2).
-double log_ibeta_cf(double a, double b, double x, double logx, double log1mx, double lbeta) {
-  const double tiny = 1e-300, eps = 1e-16;
-  const double qab = a + b, qap = a + 1.0, qam = a - 1.0;
-  double c = 1.0, d = 1.0 - qab * x / qap;
-  if (fabs(d) < tiny) d = tiny;
-  d = 1.0 / d;
-  double h = d;
-  for (int m = 1; m <= 10000; m++) {
-    const double m2 = 2.0 * m;
-    double aa = m * (b - m) * x / ((qam + m2) * (a + m2));
-    d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
-    c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
-    d = 1.0 / d;
-    h *= d * c;
-    aa = -(a + m) * (qab + m) * x / ((a + m2) * (qap + m2));
-    d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
-    c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
-    d = 1.0 / d;
-    const double del = d * c;
-    h *= del;
-    if (fabs(del - 1.0) < eps) break;
-  }
-  return a * logx + b * log1mx - lbeta - log(a) + log(h);
-}
-
-// -pbeta(x, a, b, lower.tail = FALSE, log.p = TRUE), 0 < x < 1
-double neg_log_upper_beta(double x, double a, double b, double lbeta) {
-  const double logx = log(x), log1mx = log1p(-x);
-  const double y = 1.0 - x;
-  if (y < (b + 1.0) / (a + b + 2.0)) return -log_ibeta_cf(b, a, y, log1mx, logx, lbeta);  // upper tail directly: I_{1-x}(b, a)
-  const double lp = log_ibeta_cf(a, b, x, logx, log1mx, lbeta);                              // lower tail, then complement
-  return -log1p(-exp(lp));
-}
-
 struct KeyHash {
   size_t operator()(const std::pair<int64_t, int64_t>& k) const {
     uint64_t h = (uint64_t)k.first * 0x9E3779B97F4A7C15ull ^ ((uint64_t)k.second + 0x7F4A7C15ull + ((uint64_t)k.first << 6));
@@ -323,6 +286,17 @@ struct KeyHash {
     return (size_t)h;
   }
 };
+
+// sr_links_red = srp_max > srp_cutoff; sr_links_ARACNE_check = MI >= min(sr_links_red$MI)  (:494-495), over the df rows
+// of S, whose MI are MI[S.row[i]].
+void select_red_chk(SrPostPriv& S, const double* MI, double srp_cutoff) {
+  const int64_t ndf = (int64_t)S.row.size();
+  double min_mi = INFINITY;
+  for (int64_t i = 0; i < ndf; i++)
+    if (S.srp[i] > srp_cutoff) { S.red.push_back(i); min_mi = std::min(min_mi, MI[S.row[i]]); }
+  for (int64_t i = 0; i < ndf; i++)
+    if (MI[S.row[i]] >= min_mi) S.chk.push_back(i);
+}
 
 }  // namespace
 
@@ -371,48 +345,30 @@ int beta_fit(SrPostPriv& S, int32_t c, int64_t npos, double s1, double s2, doubl
   return 0;
 }
 
-double lbeta_fn(double a, double b) {
-  int sg;
-  return lgamma_r(a, &sg) + lgamma_r(b, &sg) - lgamma_r(a + b, &sg);
-}
-
 // Links seen from two clusters: one row per distinct link, the one with the larger srp_max; groups in order of first
-// appearance, first maximum wins (:474-483, data.table `.I[which.max(srp_max)], by = keys`).  Then
-// sr_links_red = srp_max > srp_cutoff; sr_links_ARACNE_check = MI >= min(sr_links_red$MI)  (:494-495).
-// `cols` are link columns addressed by the entries of dup_at / df_at (rows of the full table on the host path, positions
-// in the gathered df table on the device path); dup_row are the rows of the full table that go into S.row.
-void dedup_and_select(SrPostPriv& S, const LinkCols& cols, const std::vector<int64_t>& dup_row, const std::vector<int64_t>& dup_at,
-                      const std::vector<int32_t>& dup_c, const std::vector<double>& dup_srp, std::vector<int64_t>& df_at, double srp_cutoff) {
-  if (!dup_row.empty()) {
-    struct Grp { int64_t first, best; };
-    std::unordered_map<std::pair<int64_t, int64_t>, std::vector<int64_t>, KeyHash> index;  // (pos1, pos2) -> groups
-    index.reserve(dup_row.size());
-    std::vector<Grp> groups;
-    groups.reserve(dup_row.size());
-    auto same = [&](int64_t a, int64_t b) {
-      return cols.pos1[a] == cols.pos1[b] && cols.pos2[a] == cols.pos2[b] && cols.clust1[a] == cols.clust1[b] &&
-             cols.clust2[a] == cols.clust2[b] && cols.len[a] == cols.len[b] && cols.MI[a] == cols.MI[b];
-    };
-    for (int64_t k = 0; k < (int64_t)dup_row.size(); k++) {
-      const int64_t r = dup_at[k];
-      auto& lst = index[{(int64_t)cols.pos1[r], (int64_t)cols.pos2[r]}];
-      int64_t g = -1;
-      for (int64_t gi : lst) if (same(dup_at[groups[gi].first], r)) { g = gi; break; }
-      if (g < 0) { lst.push_back((int64_t)groups.size()); groups.push_back({k, k}); }
-      else if (dup_srp[k] > dup_srp[groups[g].best]) groups[g].best = k;
-    }
-    const bool separate = (&df_at != &S.row);
-    for (const Grp& g : groups) {
-      S.row.push_back(dup_row[g.best]); S.clust_c.push_back(dup_c[g.best]); S.srp.push_back(dup_srp[g.best]);
-      if (separate) df_at.push_back(dup_at[g.best]);
-    }
+// appearance, first maximum wins (:474-483, data.table `.I[which.max(srp_max)], by = keys`).
+std::vector<int64_t> dedup(const ldw_links& L, const std::vector<int64_t>& at, const std::vector<double>& srp) {
+  struct Grp { int64_t first, best; };
+  std::unordered_map<std::pair<int64_t, int64_t>, std::vector<int64_t>, KeyHash> index;  // (pos1, pos2) -> groups
+  index.reserve(at.size());
+  std::vector<Grp> groups;
+  groups.reserve(at.size());
+  auto same = [&](int64_t a, int64_t b) {
+    return L.pos1[a] == L.pos1[b] && L.pos2[a] == L.pos2[b] && L.clust1[a] == L.clust1[b] && L.clust2[a] == L.clust2[b] &&
+           L.len[a] == L.len[b] && L.MI[a] == L.MI[b];
+  };
+  for (int64_t k = 0; k < (int64_t)at.size(); k++) {
+    const int64_t r = at[k];
+    auto& lst = index[{(int64_t)L.pos1[r], (int64_t)L.pos2[r]}];
+    int64_t g = -1;
+    for (int64_t gi : lst) if (same(at[groups[gi].first], r)) { g = gi; break; }
+    if (g < 0) { lst.push_back((int64_t)groups.size()); groups.push_back({k, k}); }
+    else if (srp[k] > srp[groups[g].best]) groups[g].best = k;
   }
-  const int64_t ndf = (int64_t)S.row.size();
-  double min_mi = INFINITY;
-  for (int64_t i = 0; i < ndf; i++)
-    if (S.srp[i] > srp_cutoff) { S.red.push_back(i); min_mi = std::min(min_mi, cols.MI[df_at[i]]); }
-  for (int64_t i = 0; i < ndf; i++)
-    if (cols.MI[df_at[i]] >= min_mi) S.chk.push_back(i);
+  std::vector<int64_t> win;
+  win.reserve(groups.size());
+  for (const Grp& g : groups) win.push_back(g.best);
+  return win;
 }
 
 void publish(SrPostPriv& S, int32_t nclust, ldw_sr_post* out) {
@@ -424,6 +380,23 @@ void publish(SrPostPriv& S, int32_t nclust, ldw_sr_post* out) {
   out->fit_off = S.fit_off.data(); out->fit_len = S.fit_len.data(); out->fit_q95 = S.fit_q95.data(); out->fit_val = S.fit_val.data();
   out->coef = S.coef.data(); out->shape = S.shape.data(); out->start = S.start.data();
   out->n_pos = S.n_pos.data(); out->nm_evals = S.nm_evals.data(); out->nm_fail = S.nm_fail.data();
+}
+
+int check_groups(const std::vector<int64_t>& goff, int32_t nclust, int64_t nl) {
+  for (int32_t c = 1; c <= nclust; c++)
+    if (goff[(int64_t)c * nl] == goff[(int64_t)(c - 1) * nl])
+      return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d holds no short-range link with 0 < len < sr_dist", (int)c);
+  return 0;
+}
+
+int check_residuals(int bad_c) {
+  if (bad_c) return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d: values must be in [0-1] to fit a beta distribution", bad_c);
+  return 0;
+}
+
+int check_npos(int32_t c, int64_t npos) {
+  if (npos < 2) return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d has fewer than two links above the fitted decay", (int)c);
+  return 0;
 }
 
 }  // namespace ldwpost
@@ -451,26 +424,17 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
   // R/computePairwiseMI.R:372-376), in a fixed number of contiguous pieces so that the results do not depend on the
   // number of host threads.
   PhaseTimer tm;
-  auto member = [&](int64_t i, int32_t& ca, int32_t& cb) -> bool {  // filters of :417-419; clusters the link is listed under
-    const int32_t l = sr->len[i];
-    if (!(l > 0 && (double)l < sr_dist)) return false;
-    ca = sr->clust1[i]; cb = sr->clust2[i];
-    if (ca < 1 || ca > nclust) ca = 0;
-    if (cb < 1 || cb > nclust || cb == ca) cb = 0;
-    return (ca | cb) != 0;
-  };
-  // ---- longest length present (sizes the histograms): len < sr_dist bounds it unless sr_dist is huge ----
-  int32_t maxlen = 0;
-  if (sr_dist <= (double)(1 << 18)) {
-    maxlen = (int32_t)std::max(0.0, ceil(sr_dist) - 1.0);
-  } else {
+  // ---- longest length present (sizes the histograms) ----
+  int32_t maxlen = ldwpost::max_len_bound(sr_dist);
+  if (maxlen < 0) {
+    maxlen = 0;
     const int64_t P0 = 256, p0sz = (N + P0 - 1) / P0;
     std::vector<int32_t> mx0(P0, 0);
     parallel_dynamic(P0, [&](int64_t k) {
       int32_t ml = 0;
       for (int64_t i = k * p0sz; i < std::min(N, (k + 1) * p0sz); i++) {
-        int32_t ca, cb;
-        if (member(i, ca, cb)) ml = std::max(ml, sr->len[i]);
+        int32_t ca, cb, l;
+        if (ldwpost::member(*sr, i, sr_dist, nclust, ca, cb, l)) ml = std::max(ml, l);
       }
       mx0[k] = ml;
     });
@@ -490,9 +454,8 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
     std::vector<int32_t>& h = hist[k];
     h.assign((size_t)G, 0);
     for (int64_t i = k * bsz; i < std::min(N, (k + 1) * bsz); i++) {
-      int32_t ca, cb;
-      if (!member(i, ca, cb)) continue;
-      const int64_t l = sr->len[i];
+      int32_t ca, cb, l;
+      if (!ldwpost::member(*sr, i, sr_dist, nclust, ca, cb, l)) continue;
       if (ca) h[(ca - 1) * nl + l]++;
       if (cb) h[(cb - 1) * nl + l]++;
     }
@@ -500,9 +463,7 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
   std::vector<int64_t> gcount((size_t)G, 0), goff((size_t)G + 1, 0);
   for (int64_t k = 0; k < B; k++) for (int64_t g = 0; g < G; g++) gcount[g] += hist[k][g];
   for (int64_t g = 0; g < G; g++) goff[g + 1] = goff[g] + gcount[g];
-  for (int32_t c = 1; c <= nclust; c++)
-    if (goff[(int64_t)c * nl] == goff[(int64_t)(c - 1) * nl])
-      return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d holds no short-range link with 0 < len < sr_dist", (int)c);
+  LDW_TRY(ldwpost::check_groups(goff, nclust, nl));
   std::vector<int64_t> glist;                                   // non-empty groups, cluster-major, ascending length
   for (int64_t g = 0; g < G; g++) if (gcount[g] > 0) glist.push_back(g);
   std::vector<double> gq((size_t)glist.size());
@@ -535,9 +496,8 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
     parallel_dynamic(B, [&](int64_t k) {
       int64_t* cu = bcur.data() + (size_t)k * NB;
       for (int64_t i = k * bsz; i < std::min(N, (k + 1) * bsz); i++) {
-        int32_t cc[2];
-        if (!member(i, cc[0], cc[1])) continue;
-        const int64_t l = sr->len[i];
+        int32_t cc[2], l;
+        if (!ldwpost::member(*sr, i, sr_dist, nclust, cc[0], cc[1], l)) continue;
         const double v = sr->MI[i];
         for (int q = 0; q < 2; q++) {
           if (!cc[q]) continue;
@@ -566,9 +526,7 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
   if (int rc = ldwpost::decay_fits(*S, nclust, nl, glist, gq)) return rc;
   tm.lap("decay fits", 0);
 
-  // ---- residuals above the fit (:448-450).  `mean_dist[sr_links_t$len]` subscripts the fitted values with the VALUE of
-  //      len (position in maxvls), which is the group of that length only when no shorter length is missing; a length
-  //      beyond the number of groups gives NA and the link drops out of which(diff > 0).  Reproduced as is. ----
+  // ---- residuals above the fit (:448-450), the fitted values subscripted by the value of len (sr_stats.cuh) ----
   const int64_t R = std::max<int64_t>(1, std::min<int64_t>(256, (N + kChunk - 1) / kChunk));
   const int64_t rsz = (N + R - 1) / R;
   const int C1 = nclust + 1;
@@ -577,19 +535,13 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
   std::vector<std::vector<int64_t>> lrow((size_t)R * C1);      // per piece and cluster: links above the fit, in scan order
   std::vector<std::vector<double>> lx((size_t)R * C1);
   std::atomic<int> bad(0);
-  auto residual = [&](int64_t i, int32_t c, double& d) -> bool {
-    const int64_t l = sr->len[i];
-    if (l > S->fit_off[c] - S->fit_off[c - 1]) return false;
-    d = sr->MI[i] - S->fit_val[S->fit_off[c - 1] + l - 1];
-    return d > 0;
-  };
   parallel_dynamic(R, [&](int64_t k) {
     for (int64_t i = k * rsz; i < std::min(N, (k + 1) * rsz); i++) {
-      int32_t cc[2];
-      if (!member(i, cc[0], cc[1])) continue;
+      int32_t cc[2], l;
+      if (!ldwpost::member(*sr, i, sr_dist, nclust, cc[0], cc[1], l)) continue;
       for (int q = 0; q < 2; q++) {
         double d;
-        if (!cc[q] || !residual(i, cc[q], d)) continue;
+        if (!cc[q] || !ldwpost::residual(S->fit_val.data(), S->fit_off.data(), cc[q], l, sr->MI[i], d)) continue;
         if (d > 1) bad.store(cc[q]);
         const size_t o = (size_t)k * C1 + cc[q];
         lrow[o].push_back(i); lx[o].push_back(d);
@@ -598,13 +550,13 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
     }
     for (int c = 1; c <= nclust; c++) pcnt[(size_t)(k + 1) * C1 + c] = (int64_t)lrow[(size_t)k * C1 + c].size();
   });
-  if (bad.load()) return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d: values must be in [0-1] to fit a beta distribution", bad.load());
+  LDW_TRY(ldwpost::check_residuals(bad.load()));
   for (int64_t k = 0; k < R; k++) for (int c = 1; c <= nclust; c++) pcnt[(size_t)(k + 1) * C1 + c] += pcnt[(size_t)k * C1 + c];
   std::vector<std::vector<int64_t>> prow(C1);
   std::vector<std::vector<double>> px(C1);
   for (int32_t c = 1; c <= nclust; c++) {
     const int64_t npos = pcnt[(size_t)R * C1 + c];
-    if (npos < 2) return ldw::set_error(LDW_ERR_ARG, "ldw_sr_postprocess: cluster %d has fewer than two links above the fitted decay", (int)c);
+    LDW_TRY(ldwpost::check_npos(c, npos));
     prow[c].resize((size_t)npos);
     px[c].resize((size_t)npos);
   }
@@ -642,12 +594,11 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
     if (int rc = ldwpost::beta_fit(*S, c, npos, (double)s1, (double)s2, mean, v, par)) return rc;
     tm.lap("beta fit", c);
     // ---- srp = -pbeta(x, shape1, shape2, lower.tail = F, log.p = T)  (:453) ----
-    int sg;
-    const double lbeta = lgamma_r(par[0], &sg) + lgamma_r(par[1], &sg) - lgamma_r(par[0] + par[1], &sg);
+    const double lbeta = ldwpost::lbeta_fn(par[0], par[1]);
     std::vector<double> psrp(npos);
     parallel_dynamic(pchunks, [&](int64_t k) {
       const int64_t lo = k * kChunk, hi = std::min(npos, lo + kChunk);
-      for (int64_t i = lo; i < hi; i++) psrp[i] = x[i] < 1.0 ? neg_log_upper_beta(x[i], par[0], par[1], lbeta) : INFINITY;
+      for (int64_t i = lo; i < hi; i++) psrp[i] = x[i] < 1.0 ? ldwpost::neg_log_upper_beta(x[i], par[0], par[1], lbeta) : INFINITY;
     });
     tm.lap("srp", c);
     // ---- same-cluster links go to sr_links_df, links between clusters to duplink_df (:460-468) ----
@@ -662,8 +613,8 @@ extern "C" int ldw_sr_postprocess(const ldw_links* sr, int32_t nclust, double sr
     std::vector<double>().swap(px[c]);
   }
   tm.lap("(last cluster's append)", nclust);
-  ldwpost::LinkCols cols{sr->pos1, sr->pos2, sr->clust1, sr->clust2, sr->len, sr->MI};
-  ldwpost::dedup_and_select(*S, cols, dup_row, dup_row, dup_c, dup_srp, S->row, srp_cutoff);
+  for (int64_t k : ldwpost::dedup(*sr, dup_row, dup_srp)) { S->row.push_back(dup_row[k]); S->clust_c.push_back(dup_c[k]); S->srp.push_back(dup_srp[k]); }
+  select_red_chk(*S, sr->MI, srp_cutoff);
 
   tm.lap("dedup + red/chk", 0);
   ldwpost::publish(*S, nclust, out);
@@ -689,11 +640,10 @@ extern "C" int ldw_neg_log_pbeta_upper(const double* x, int64_t n, double shape1
   return guarded("ldw_neg_log_pbeta_upper", [&]() -> int {
   if (n < 0 || (n > 0 && (!x || !out))) return ldw::set_error(LDW_ERR_ARG, "ldw_neg_log_pbeta_upper: bad argument");
   if (!(shape1 > 0 && shape2 > 0)) return ldw::set_error(LDW_ERR_ARG, "ldw_neg_log_pbeta_upper: shapes must be positive");
-  int sg;
-  const double lbeta = lgamma_r(shape1, &sg) + lgamma_r(shape2, &sg) - lgamma_r(shape1 + shape2, &sg);
+  const double lbeta = ldwpost::lbeta_fn(shape1, shape2);
   parallel_dynamic((n + kChunk - 1) / kChunk, [&](int64_t k) {
     for (int64_t i = k * kChunk; i < std::min(n, (k + 1) * kChunk); i++)
-      out[i] = x[i] <= 0 ? 0.0 : x[i] >= 1 ? INFINITY : neg_log_upper_beta(x[i], shape1, shape2, lbeta);
+      out[i] = x[i] <= 0 ? 0.0 : x[i] >= 1 ? INFINITY : ldwpost::neg_log_upper_beta(x[i], shape1, shape2, lbeta);
   });
   return 0;
   });
